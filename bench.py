@@ -26,6 +26,13 @@ Beside the headline the line carries (each outside the headline's timed region, 
             issue (DESIGN.md "Roofline"), peak = best IMAD.WIDE.U32 rate measured by probe kernels in the same run;
             an `hbm` sub-object shows HBM is three orders of magnitude from binding
   cpu_baseline  oracle (C restatement of the reference path; the Nim toolchain is absent) on a bounded sample
+
+--dump-outputs DIR writes what the last timed step of the headline committed (rank 0's part at N > 1) as float64 .npy
+files, each field element as 8 little-endian 32-bit limbs (exact in float64), so that two builds can be compared output
+for output: slot_root, block_hashes and cell_hashes, each layer whole up to 2^18 nodes and otherwise a seeded sample of
+32-node windows, with the global node numbers beside it (<name>_index.npy).  Under 40 MB whatever the slot size.
+
+Nothing is written into the source tree (it may be read-only): the host-tuned oracle build goes to a temporary directory.
 """
 from __future__ import annotations
 
@@ -98,6 +105,41 @@ def synthetic_bytes_host(seed: int, first_word: int, n_bytes: int):
         z = (z ^ (z >> np.uint64(27))) * np.uint64(0x94d049bb133111eb)
         z = z ^ (z >> np.uint64(31))
     return z.view(np.uint8)
+
+
+# ---------------------------------------------------------------------------------------------------------------
+# --dump-outputs
+
+DUMP_MAX_NODES = 1 << 18                     # per layer: 2^18 nodes x 8 limbs x 8 bytes = 16 MiB (+ 2 MiB of node numbers)
+DUMP_WINDOW = 32                             # sampled layers are read in windows of 32 nodes (one block's cells)
+
+
+def dump_layer(slot, tree: int, level: int, first: int, count: int, rng):
+    """(node numbers, (n, 8) float64 limbs) of nodes [first, first + count) of one retained layer: all of them up to
+    DUMP_MAX_NODES, else a seeded sample of DUMP_WINDOW-node windows"""
+    import numpy as np
+    if count <= DUMP_MAX_NODES:
+        windows = [(first, count)]
+    else:
+        starts = np.sort(rng.choice(count // DUMP_WINDOW, DUMP_MAX_NODES // DUMP_WINDOW, replace=False))
+        windows = [(first + int(s) * DUMP_WINDOW, DUMP_WINDOW) for s in starts]
+    idx = np.concatenate([np.arange(f, f + n, dtype=np.float64) for f, n in windows])
+    raw = b"".join(int(v).to_bytes(32, "little") for f, n in windows for v in slot.read_layer(tree, level, f, n))
+    return idx, np.frombuffer(raw, dtype="<u4").reshape(-1, 8).astype(np.float64)
+
+
+def dump_outputs(out_dir: str, slot, first_block: int, n_blocks: int) -> None:
+    """the slot's root, its block hashes and its cell hashes (of blocks [first_block, first_block + n_blocks)) as .npy"""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    rng = np.random.default_rng(SEED)
+    cells_per_block = BLOCK // CELL
+    out = {"slot_root": np.frombuffer(slot.root.to_bytes(32, "little"), dtype="<u4").reshape(1, 8).astype(np.float64)}
+    out["block_hashes_index"], out["block_hashes"] = dump_layer(slot, 1, 0, first_block, n_blocks, rng)
+    out["cell_hashes_index"], out["cell_hashes"] = dump_layer(slot, 0, 0, first_block * cells_per_block, n_blocks * cells_per_block, rng)
+    for name, arr in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), arr)
+    print(f"dumped {', '.join(out)} ({sum(a.nbytes for a in out.values()) / 2**20:.1f} MiB) to {out_dir}", file=sys.stderr)
 
 
 def host_threads() -> int:
@@ -251,7 +293,11 @@ def main() -> None:
     ap.add_argument("--config5-slots", type=int, default=250)
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed as .npy files under DIR")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    sys.dont_write_bytecode = True              # nothing is written into the tree, not even __pycache__
     if args.impl == "reference":
         return run_reference(args)
 
@@ -296,15 +342,20 @@ def main() -> None:
             dist.barrier()
         torch.cuda.synchronize()
 
+    kept = []                                         # --dump-outputs: the latest step's slot, read after the timed region
+
     def commit_resident():
         if world == 1:
             slot = ctx.slot_commit_dev(d_slot.data_ptr(), n_bytes, CELL, BLOCK)
-            root = slot.root                          # 32-byte D2H, synchronises the stream
+        else:
+            slot = ctx.slot_commit_sharded_dev(comm, d_slot.data_ptr(), n_bytes, CELL, BLOCK, first_block, n_total_blocks, top_level)
+        root = slot.root                              # 32-byte D2H, synchronises the stream
+        if args.dump_outputs:                         # free the previous step's slot instead: still one free per step
+            for s in kept:
+                s.free()
+            kept[:] = [slot]
+        else:
             slot.free()
-            return root
-        sh = ctx.slot_commit_sharded_dev(comm, d_slot.data_ptr(), n_bytes, CELL, BLOCK, first_block, n_total_blocks, top_level)
-        root = sh.root
-        sh.free()
         return root
 
     def timed(fn, steps):
@@ -345,6 +396,10 @@ def main() -> None:
     total_bytes = n_total_blocks * BLOCK
     value = total_bytes * args.steps / ev_s / 1e9
     perms_step = total_perms(n_total_blocks)
+    if kept:
+        if rank == 0:
+            dump_outputs(args.dump_outputs, kept[0], first_block, my_blocks)
+        kept.pop().free()
 
     # ---- dominant kernel alone (roofline) ----
     n_cells = n_bytes // CELL

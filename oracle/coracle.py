@@ -4,9 +4,12 @@ Field elements are python ints at this level; they cross into C as 32-byte littl
 """
 from __future__ import annotations
 
+import atexit
 import ctypes as C
 import os
+import shutil
 import subprocess
+import tempfile
 from typing import List, Optional, Sequence, Tuple
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
@@ -39,14 +42,15 @@ def build(force: bool = False) -> str:
 
 def use_native() -> bool:
     """Switch to a build tuned for THIS machine (-O3 -march=native), compiled here and now; used by bench.py's CPU legs so
-    that the reported baseline is not handicapped by generic code.  Returns False (and keeps the portable build) if the
-    compiler is missing or the build fails."""
+    that the reported baseline is not handicapped by generic code.  The library goes to a fresh temporary directory
+    (removed at exit), so the source tree may be read-only.  Returns False (and keeps the portable build) if the compiler
+    is missing or the build fails."""
     global _SO, _lib
-    native = os.path.join(_HERE, "build", "libcodex_oracle_native.so")
+    out_dir = tempfile.mkdtemp(prefix="codex_oracle_native_")
+    atexit.register(shutil.rmtree, out_dir, True)
+    native = os.path.join(out_dir, "libcodex_oracle_native.so")
     try:
-        if os.path.exists(native):
-            os.remove(native)                      # never trust a copy that travelled from another machine
-        subprocess.run(["make", "-C", _HERE, "-s", "native"], check=True, capture_output=True)
+        subprocess.run(["make", "-C", _HERE, "-s", "native", "BUILD=" + out_dir], check=True, capture_output=True)
         C.CDLL(native)
     except Exception:
         return False
