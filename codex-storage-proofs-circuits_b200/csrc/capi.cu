@@ -35,7 +35,7 @@ struct cdx_ctx {
   cudaStream_t stream = nullptr;       // compute
   cudaStream_t copy_stream = nullptr;  // H2D staging for *_host entry points
   cudaStream_t copy_stream2 = nullptr; // second H2D stream: the copies of consecutive tiles of a pinned slot alternate (two in flight)
-  cudaStream_t stream2 = nullptr;      // second compute stream: odd tiles of a host-resident slot (kernels overlap at the tile seams)
+  cudaStream_t stream2 = nullptr;      // second compute stream: odd tiles of a streamed slot (kernels overlap at the tile seams)
   cudaEvent_t ev_join = nullptr;
   cudaEvent_t ev_copied[CDX_MAX_STAGE] = {nullptr, nullptr, nullptr, nullptr};
   cudaEvent_t ev_consumed[CDX_MAX_STAGE] = {nullptr, nullptr, nullptr, nullptr};
@@ -202,14 +202,24 @@ extern "C" int cdx_ctx_create(int device, cdx_ctx** out) {
   return CDX_OK;
 }
 
-extern "C" void cdx_ctx_destroy(cdx_ctx* ctx) {
-  if (!ctx) return;
-  cudaSetDevice(ctx->device);
+// The staging ring comes from cudaMalloc, not from the stream-ordered pool: without guard bands it goes back through cudaFree.
+static void release_stage(cdx_ctx* ctx) {
   for (int i = 0; i < CDX_MAX_STAGE; ++i) {
     if (ctx->d_stage[i]) {
       if (guard_enabled()) dev_free(ctx->d_stage[i], ctx->stream);
       else cudaFree(ctx->d_stage[i]);
     }
+    ctx->d_stage[i] = nullptr;
+  }
+  ctx->stage_bytes = 0;
+  ctx->stage_count = 0;
+}
+
+extern "C" void cdx_ctx_destroy(cdx_ctx* ctx) {
+  if (!ctx) return;
+  cudaSetDevice(ctx->device);
+  release_stage(ctx);
+  for (int i = 0; i < CDX_MAX_STAGE; ++i) {
     if (ctx->ev_copied[i]) cudaEventDestroy(ctx->ev_copied[i]);
     if (ctx->ev_consumed[i]) cudaEventDestroy(ctx->ev_consumed[i]);
   }
@@ -766,22 +776,12 @@ extern "C" int cdx_slot_commit_dev(cdx_ctx* ctx, const void* d_data, size_t n_by
   return CDX_OK;
 }
 
-static void stage_free(cdx_ctx* ctx, void* p) {
-  if (guard_enabled()) dev_free(p, ctx->stream);
-  else cudaFree(p);
-}
-
 static int ensure_stage(cdx_ctx* ctx, size_t bytes, int count = 2) {
   if (ctx->stage_bytes >= bytes && ctx->stage_count >= count) return CDX_OK;
   const size_t want_bytes = bytes > ctx->stage_bytes ? bytes : ctx->stage_bytes;
   const int want_count = count > ctx->stage_count ? count : ctx->stage_count;
   CU_TRY(ctx, cudaDeviceSynchronize());                       // earlier calls may still be reading the old tiles
-  for (int i = 0; i < CDX_MAX_STAGE; ++i) {
-    if (ctx->d_stage[i]) stage_free(ctx, ctx->d_stage[i]);
-    ctx->d_stage[i] = nullptr;
-  }
-  ctx->stage_bytes = 0;
-  ctx->stage_count = 0;
+  release_stage(ctx);
   for (int i = 0; i < want_count; ++i) CU_TRY(ctx, dev_alloc(&ctx->d_stage[i], want_bytes, ctx->stream, false));
   ctx->stage_bytes = want_bytes;
   ctx->stage_count = want_count;
@@ -789,9 +789,13 @@ static int ensure_stage(cdx_ctx* ctx, size_t bytes, int count = 2) {
 }
 
 // ---- cell-hash pipelines: slot bytes that are not resident in HBM -------------------------------------------------
-// Each of the three streams its source through two device tiles and leaves the cell hashes in d_hashes.  They queue work
-// on ctx->stream / ctx->stream2 / ctx->copy_stream and return with ctx->stream ordered after all of it (no host sync);
-// the caller continues on ctx->stream.
+// Every source that is not in HBM (pinned or pageable host memory, a file, generated bytes) reaches the cell sponge
+// through run_tiles.  The slot is cut into tiles of whole blocks.  Tile t is produced into staging buffer t % n_bufs and
+// hashed on compute stream t & 1: two compute streams let the sponge kernels of consecutive tiles overlap at the seams
+// (the tail of one fills up with the head of the next).  Each buffer is reused strictly in order: the producer of tile t
+// waits for the sponge of tile t - n_bufs, and the sponge of tile t waits for its producer.  The pipelines differ only
+// in their tile sizes, their number of buffers and their producer.  They return with ctx->stream ordered after all of
+// their work (no host sync); the caller continues on ctx->stream.
 typedef std::function<void(uint8_t* dst, uint64_t offset, size_t len)> ChunkFill;
 
 static void drain_streams(cdx_ctx* ctx) {
@@ -801,7 +805,89 @@ static void drain_streams(cdx_ctx* ctx) {
   cudaStreamSynchronize(ctx->stream);
 }
 
-// Pinned (or otherwise DMA-able) host memory: the copy of tile t+1 (copy stream) overlaps the cell sponge of tile t.
+// An open slot data file as a ChunkFill.  A read error is not an end of file: EINTR is retried, anything else is
+// recorded (the fill runs on worker threads) and fails the commit; only a true EOF zero-fills, like the reference's
+// ignored short reads (slot.nim:64-65).
+struct FileSource {
+  int fd = -1;
+  uint64_t base = 0;
+  std::atomic<int> io_errno{0};
+  ChunkFill fill;
+  ~FileSource() {
+    if (fd >= 0) close(fd);
+  }
+  bool open_path(const char* path, uint64_t base_offset) {
+    fd = open(path, O_RDONLY);
+    base = base_offset;
+    fill = [this](uint8_t* dst, uint64_t off, size_t len) {
+      size_t pos = 0;
+      while (pos < len) {
+        const ssize_t got = pread(fd, dst + pos, len - pos, (off_t)(base + off + pos));
+        if (got < 0) {
+          if (errno == EINTR) continue;
+          int expected = 0;
+          io_errno.compare_exchange_strong(expected, errno);
+          break;
+        }
+        if (got == 0) break;
+        pos += (size_t)got;
+      }
+      if (pos < len) memset(dst + pos, 0, len - pos);
+    };
+    return fd >= 0;
+  }
+};
+
+// tile sizes in blocks: `head`, then `tile` until n_blocks are covered; the last tile is clipped to what remains
+static std::vector<size_t> tile_schedule(size_t n_blocks, const std::vector<size_t>& head, size_t tile) {
+  std::vector<size_t> tiles;
+  for (size_t done = 0; done < n_blocks; done += tiles.back()) {
+    const size_t want = tiles.size() < head.size() ? head[tiles.size()] : tile;
+    tiles.push_back(n_blocks - done < want ? n_blocks - done : want);
+  }
+  return tiles;
+}
+
+// queues the bytes of blocks [first, first + nb), which make up tile t, into the staging buffer dst on stream st
+typedef std::function<int(int t, size_t first, size_t nb, uint8_t* dst, cudaStream_t st)> TileProducer;
+
+// Tiles with an even index are produced on `even`, those with an odd index on `odd`; a null stream produces the tile on
+// its compute stream.  Only these streams and ctx->stream2 are ordered after the caller's earlier work on ctx->stream: a
+// copy stream held up for nothing would also hold up upload_table, whose next call waits on the host for the last one.
+static int run_tiles(cdx_ctx* ctx, const std::vector<size_t>& tiles, int n_bufs, cudaStream_t even, cudaStream_t odd, size_t cell_size,
+                     size_t block_size, const TileProducer& produce, uint8_t* d_hashes) {
+  CU_TRY(ctx, cudaEventRecord(ctx->ev_join, ctx->stream));              // d_hashes was allocated on ctx->stream, and
+  CU_TRY(ctx, cudaStreamWaitEvent(ctx->stream2, ctx->ev_join, 0));      // earlier work on it may still read the buffers
+  if (even) CU_TRY(ctx, cudaStreamWaitEvent(even, ctx->ev_join, 0));
+  if (odd && odd != even) CU_TRY(ctx, cudaStreamWaitEvent(odd, ctx->ev_join, 0));
+  const size_t cpb = block_size / cell_size;
+  size_t first = 0;
+  for (int t = 0; t < (int)tiles.size(); ++t) {
+    const int b = t % n_bufs;
+    const size_t nb = tiles[t];
+    cudaStream_t cs = (t & 1) ? ctx->stream2 : ctx->stream;
+    cudaStream_t ps = (t & 1) ? odd : even;
+    if (!ps) ps = cs;
+    if (t >= n_bufs) CU_TRY(ctx, cudaStreamWaitEvent(ps, ctx->ev_consumed[b], 0));
+    int rc = produce(t, first, nb, (uint8_t*)ctx->d_stage[b], ps);
+    if (rc) return rc;
+    if (ps != cs) {
+      CU_TRY(ctx, cudaEventRecord(ctx->ev_copied[b], ps));
+      CU_TRY(ctx, cudaStreamWaitEvent(cs, ctx->ev_copied[b], 0));
+    }
+    rc = launch_hash_cells(ctx, ctx->d_stage[b], nb * cpb, cell_size, d_hashes + 32 * first * cpb, cs);
+    if (rc) return rc;
+    CU_TRY(ctx, cudaEventRecord(ctx->ev_consumed[b], cs));
+    first += nb;
+  }
+  CU_TRY(ctx, cudaEventRecord(ctx->ev_join, ctx->stream2));             // the caller's trees run on ctx->stream after both
+  CU_TRY(ctx, cudaStreamWaitEvent(ctx->stream, ctx->ev_join, 0));       // compute streams
+  return CDX_OK;
+}
+
+// Pinned (or otherwise DMA-able) host memory: one copy per tile, on copy stream t & 1.  NS = 3 buffers and two copy
+// streams keep TWO copies in flight ahead of the sponge, which rides out a host whose PCIe/memory path is shared by eight
+// GPUs streaming at once (DESIGN.md section 7).
 static int hash_cells_pinned(cdx_ctx* ctx, const uint8_t* data, size_t n_bytes, size_t cell_size, size_t block_size, uint8_t* d_hashes) {
   const size_t n_blocks = n_bytes / block_size;
   // Tile = 256 MiB: 131 072 cells of 2 KiB, about one full wave of the cell-sponge kernel on 148 SMs (the resident
@@ -815,17 +901,6 @@ static int hash_cells_pinned(cdx_ctx* ctx, const uint8_t* data, size_t n_bytes, 
   const int NS = ctx->stage_tiles;
   int rc = ensure_stage(ctx, tile_blocks * block_size, NS);
   if (rc) return rc;
-  const size_t cpb = block_size / cell_size;
-  // Tile t lives in staging buffer t % NS, is copied on copy stream t&1 and hashed on compute stream t&1.  Two compute
-  // streams let the cell kernels of consecutive tiles overlap at the seams (the tail of one fills up with the head of the
-  // next); NS = 3 buffers and two copy streams keep TWO copies in flight ahead of the sponge, which rides out a host
-  // whose PCIe/memory path is shared by eight GPUs streaming at once (DESIGN.md section 7).  Each buffer is reused strictly
-  // in order: copy(t) waits for hash(t-NS), hash(t) waits for copy(t).
-  CU_TRY(ctx, cudaEventRecord(ctx->ev_join, ctx->stream));              // the hash buffer was allocated on stream
-  CU_TRY(ctx, cudaStreamWaitEvent(ctx->stream2, ctx->ev_join, 0));
-  CU_TRY(ctx, cudaStreamWaitEvent(ctx->copy_stream, ctx->ev_join, 0));  // and the staging tiles may still be read by earlier work on it
-  CU_TRY(ctx, cudaStreamWaitEvent(ctx->copy_stream2, ctx->ev_join, 0));
-  size_t done = 0;
   // Start of the pipeline.  The copy of tile 0 is the only one nothing overlaps, so it is short; after that the copy of
   // tile t+1 has to hide behind the sponge of tile t.  Two starts:
   //   mode 0  1/8 tile, then 7/8 (realigns with the tile grid);
@@ -835,7 +910,6 @@ static int hash_cells_pinned(cdx_ctx* ctx, const uint8_t* data, size_t n_bytes, 
   // GPU).  So the default (mode 2) decides per call from the H2D rate this context measured on its previous pinned
   // commit (two events around one full-size tile copy, read back here without waiting): gradual above 48 GB/s, else
   // mode 0; the first commit of a context uses mode 0.  CODEX_COMMIT_RAMP=0/1 pins the choice.
-  const bool ramp = n_blocks > tile_blocks && tile_blocks >= 8;
   if (ctx->rate_bytes) {
     float ms = 0.f;
     if (cudaEventElapsedTime(&ms, ctx->ev_rate[0], ctx->ev_rate[1]) == cudaSuccess && ms > 0.f) {
@@ -846,45 +920,33 @@ static int hash_cells_pinned(cdx_ctx* ctx, const uint8_t* data, size_t n_bytes, 
     }
   }
   const bool gradual = ctx->ramp_mode == 1 || (ctx->ramp_mode == 2 && ctx->h2d_gbs > 48.0);
-  size_t cur = gradual ? (tile_blocks / 4 ? tile_blocks / 4 : 1) : (tile_blocks / 8 ? tile_blocks / 8 : 1);
-  bool rate_armed = false;
-  for (int t = 0; done < n_blocks; ++t) {
-    const int b = t % NS;
-    cudaStream_t cs = (t & 1) ? ctx->stream2 : ctx->stream;
-    cudaStream_t cp = (t & 1) ? ctx->copy_stream2 : ctx->copy_stream;
-    size_t want = tile_blocks;
-    if (ramp && gradual) {
-      want = cur < tile_blocks ? cur : tile_blocks;
-      cur += cur / 4 ? cur / 4 : 1;
-    } else if (ramp) {
-      if (t == 0) want = cur;
-      else if (t == 1) want = tile_blocks - cur;
+  std::vector<size_t> head;
+  if (n_blocks > tile_blocks && tile_blocks >= 8) {
+    if (gradual) {
+      for (size_t cur = tile_blocks / 4; cur < tile_blocks; cur += cur / 4 ? cur / 4 : 1) head.push_back(cur);
+    } else {
+      head = {tile_blocks / 8, tile_blocks - tile_blocks / 8};
     }
-    const size_t nb = n_blocks - done < want ? n_blocks - done : want;
-    if (t >= NS) CU_TRY(ctx, cudaStreamWaitEvent(cp, ctx->ev_consumed[b], 0));
+  }
+  bool rate_armed = false;
+  auto copy = [&](int t, size_t first, size_t nb, uint8_t* dst, cudaStream_t cp) -> int {
     const bool measure = !rate_armed && nb == tile_blocks && t >= NS;    // a full tile in steady state (its buffer wait is already behind it)
     if (measure) CU_TRY(ctx, cudaEventRecord(ctx->ev_rate[0], cp));
-    CU_TRY(ctx, cudaMemcpyAsync(ctx->d_stage[b], data + done * block_size, nb * block_size, cudaMemcpyHostToDevice, cp));
+    CU_TRY(ctx, cudaMemcpyAsync(dst, data + first * block_size, nb * block_size, cudaMemcpyHostToDevice, cp));
     if (measure) {
       CU_TRY(ctx, cudaEventRecord(ctx->ev_rate[1], cp));
       ctx->rate_bytes = nb * block_size;
       rate_armed = true;
     }
-    CU_TRY(ctx, cudaEventRecord(ctx->ev_copied[b], cp));
-    CU_TRY(ctx, cudaStreamWaitEvent(cs, ctx->ev_copied[b], 0));
-    int hr = launch_hash_cells(ctx, ctx->d_stage[b], nb * cpb, cell_size, d_hashes + 32 * done * cpb, cs);
-    if (hr) return hr;
-    CU_TRY(ctx, cudaEventRecord(ctx->ev_consumed[b], cs));
-    done += nb;
-  }
-  CU_TRY(ctx, cudaEventRecord(ctx->ev_join, ctx->stream2));             // the caller's trees run on stream after both tile streams
-  CU_TRY(ctx, cudaStreamWaitEvent(ctx->stream, ctx->ev_join, 0));
-  return CDX_OK;
+    return CDX_OK;
+  };
+  return run_tiles(ctx, tile_schedule(n_blocks, head, tile_blocks), NS, ctx->copy_stream, ctx->copy_stream2, cell_size, block_size, copy,
+                   d_hashes);
 }
 
-// Slot bytes that are not directly DMA-able (a file, or pageable host memory -- what a Nim seq[byte] is).  Three
-// overlapped stages: host threads fill one of two pinned chunks through `fill(dst, offset, len)`, H2D of that chunk
-// into the current device tile (copy stream), cell sponge per finished tile (alternating compute streams).
+// Slot bytes that are not directly DMA-able (a file, or pageable host memory -- what a Nim seq[byte] is).  Host threads
+// fill one of two pinned chunks through `fill(dst, offset, len)` while the copy stream moves the other one into the
+// device tile; a tile is four chunks, copied on the one copy stream into two device buffers.
 static int hash_cells_staged(cdx_ctx* ctx, size_t n_bytes, size_t cell_size, size_t block_size, const ChunkFill& fill, uint8_t* d_hashes) {
   const size_t n_blocks = n_bytes / block_size;
   const size_t chunk_bytes_target = (ctx->tile_mib << 20) / 4;              // pinned chunk
@@ -906,7 +968,6 @@ static int hash_cells_staged(cdx_ctx* ctx, size_t n_bytes, size_t cell_size, siz
   }
   int rc = ensure_stage(ctx, tile_bytes);
   if (rc) return rc;
-  const size_t cpb = block_size / cell_size;
   unsigned hw = std::thread::hardware_concurrency();
   const unsigned n_thr = hw >= 16 ? 8 : (hw >= 8 ? 4 : 2);
   auto fill_chunk_parallel = [&](uint8_t* dst, uint64_t off, size_t len) {
@@ -917,41 +978,26 @@ static int hash_cells_staged(cdx_ctx* ctx, size_t n_bytes, size_t cell_size, siz
     }
     for (auto& t : thr) t.join();
   };
-  CU_TRY(ctx, cudaEventRecord(ctx->ev_join, ctx->stream));
-  CU_TRY(ctx, cudaStreamWaitEvent(ctx->stream2, ctx->ev_join, 0));
-  CU_TRY(ctx, cudaStreamWaitEvent(ctx->copy_stream, ctx->ev_join, 0));
-  size_t done_blocks = 0, chunk_no = 0;
-  const bool ramp = n_blocks > tile_blocks && tile_blocks > chunk_blocks;
-  for (int t = 0; done_blocks < n_blocks; ++t) {
-    const int b = t & 1;
-    cudaStream_t cs = b ? ctx->stream2 : ctx->stream;
-    // tile 0 is one chunk, tile 1 the other three: the sponge starts after one chunk has been filled and copied, not four
-    size_t want = tile_blocks;
-    if (ramp && t == 0) want = chunk_blocks;
-    else if (ramp && t == 1) want = tile_blocks - chunk_blocks;
-    const size_t nb = n_blocks - done_blocks < want ? n_blocks - done_blocks : want;
-    if (t >= 2) CU_TRY(ctx, cudaStreamWaitEvent(ctx->copy_stream, ctx->ev_consumed[b], 0));   // device tile b free again
+  // tile 0 is one chunk, tile 1 the other three: the sponge starts after one chunk has been filled and copied, not four
+  std::vector<size_t> head;
+  if (n_blocks > tile_blocks && tile_blocks > chunk_blocks) head = {chunk_blocks, tile_blocks - chunk_blocks};
+  size_t chunk_no = 0;
+  auto copy = [&](int, size_t first, size_t nb, uint8_t* dst, cudaStream_t cp) -> int {
     for (size_t cb = 0; cb < nb; cb += chunk_blocks, ++chunk_no) {
       const int pb = (int)(chunk_no & 1);
       const size_t cnb = nb - cb < chunk_blocks ? nb - cb : chunk_blocks;
       if (chunk_no >= 2) CU_TRY(ctx, cudaEventSynchronize(ctx->ev_h2d[pb]));                  // pinned chunk pb drained
-      fill_chunk_parallel((uint8_t*)ctx->h_pinned[pb], (uint64_t)(done_blocks + cb) * block_size, cnb * block_size);
-      CU_TRY(ctx, cudaMemcpyAsync((uint8_t*)ctx->d_stage[b] + cb * block_size, ctx->h_pinned[pb], cnb * block_size, cudaMemcpyHostToDevice,
-                                  ctx->copy_stream));
-      CU_TRY(ctx, cudaEventRecord(ctx->ev_h2d[pb], ctx->copy_stream));
+      fill_chunk_parallel((uint8_t*)ctx->h_pinned[pb], (uint64_t)(first + cb) * block_size, cnb * block_size);
+      CU_TRY(ctx, cudaMemcpyAsync(dst + cb * block_size, ctx->h_pinned[pb], cnb * block_size, cudaMemcpyHostToDevice, cp));
+      CU_TRY(ctx, cudaEventRecord(ctx->ev_h2d[pb], cp));
     }
-    CU_TRY(ctx, cudaEventRecord(ctx->ev_copied[b], ctx->copy_stream));
-    CU_TRY(ctx, cudaStreamWaitEvent(cs, ctx->ev_copied[b], 0));
-    int hr = launch_hash_cells(ctx, ctx->d_stage[b], nb * cpb, cell_size, d_hashes + 32 * done_blocks * cpb, cs);
-    if (hr) return hr;
-    CU_TRY(ctx, cudaEventRecord(ctx->ev_consumed[b], cs));
-    done_blocks += nb;
-  }
+    return CDX_OK;
+  };
+  rc = run_tiles(ctx, tile_schedule(n_blocks, head, tile_blocks), 2, ctx->copy_stream, ctx->copy_stream, cell_size, block_size, copy, d_hashes);
+  if (rc) return rc;
   // the pinned chunks are reused by the next call: their last copies must have left the host
   CU_TRY(ctx, cudaEventSynchronize(ctx->ev_h2d[0]));
   if (chunk_no >= 2) CU_TRY(ctx, cudaEventSynchronize(ctx->ev_h2d[1]));
-  CU_TRY(ctx, cudaEventRecord(ctx->ev_join, ctx->stream2));
-  CU_TRY(ctx, cudaStreamWaitEvent(ctx->stream, ctx->ev_join, 0));
   return CDX_OK;
 }
 
@@ -971,8 +1017,8 @@ static int hash_cells_host(cdx_ctx* ctx, const uint8_t* data, size_t n_bytes, si
 }
 
 // Generated slot bytes (the reference's fake data or the benchmark's counter-based bytes): the generator kernel writes a
-// device tile, the sponge reads it on the same stream; two tiles on two streams.  Nothing crosses PCIe and no slot-sized
-// buffer exists, so a 100 GiB slot costs 512 MiB of staging.  first_byte is the offset of this range inside its slot.
+// device tile on the tile's compute stream, two tiles in flight.  Nothing crosses PCIe and no slot-sized buffer exists,
+// so a 100 GiB slot costs 512 MiB of staging.  first_byte is the offset of this range inside its slot.
 static int launch_fake_cells(cdx_ctx* ctx, uint64_t seed, uint64_t first_cell, size_t n_cells, size_t cell_size, void* d_out, cudaStream_t st);
 static int launch_fill_synthetic(cdx_ctx* ctx, uint64_t seed, uint64_t first_word, size_t n_bytes, void* d_out, cudaStream_t st);
 static int generate_bytes(cdx_ctx* ctx, uint32_t kind, uint64_t seed, uint64_t first_byte, size_t n_bytes, size_t cell_size, void* d_out, cudaStream_t st) {
@@ -987,22 +1033,10 @@ static int hash_cells_generated(cdx_ctx* ctx, uint32_t kind, uint64_t seed, uint
   if (tile_blocks > n_blocks) tile_blocks = n_blocks;
   int rc = ensure_stage(ctx, tile_blocks * block_size);
   if (rc) return rc;
-  const size_t cpb = block_size / cell_size;
-  CU_TRY(ctx, cudaEventRecord(ctx->ev_join, ctx->stream));
-  CU_TRY(ctx, cudaStreamWaitEvent(ctx->stream2, ctx->ev_join, 0));
-  size_t done = 0;
-  for (int t = 0; done < n_blocks; ++t) {
-    cudaStream_t cs = (t & 1) ? ctx->stream2 : ctx->stream;           // tile b is only ever touched on stream b: ordered by the stream
-    const size_t nb = n_blocks - done < tile_blocks ? n_blocks - done : tile_blocks;
-    rc = generate_bytes(ctx, kind, seed, first_byte + done * block_size, nb * block_size, cell_size, ctx->d_stage[t & 1], cs);
-    if (rc) return rc;
-    rc = launch_hash_cells(ctx, ctx->d_stage[t & 1], nb * cpb, cell_size, d_hashes + 32 * done * cpb, cs);
-    if (rc) return rc;
-    done += nb;
-  }
-  CU_TRY(ctx, cudaEventRecord(ctx->ev_join, ctx->stream2));
-  CU_TRY(ctx, cudaStreamWaitEvent(ctx->stream, ctx->ev_join, 0));
-  return CDX_OK;
+  auto generate = [&](int, size_t first, size_t nb, uint8_t* dst, cudaStream_t st) {
+    return generate_bytes(ctx, kind, seed, first_byte + first * block_size, nb * block_size, cell_size, dst, st);
+  };
+  return run_tiles(ctx, tile_schedule(n_blocks, {}, tile_blocks), 2, nullptr, nullptr, cell_size, block_size, generate, d_hashes);
 }
 
 // where the bytes of a slot (or of a block range of one) come from
@@ -1087,35 +1121,16 @@ extern "C" int cdx_slot_commit_file(cdx_ctx* ctx, const char* path, uint64_t off
   *out = nullptr;
   int rc = check_shape(ctx, n_bytes, cell_size, block_size);
   if (rc) return rc;
-  const int fd = open(path, O_RDONLY);
-  if (fd < 0) return fail(ctx, CDX_ERR_ARG, "cannot open slot data file `%s`", path);
-  // A read error is not an end of file: EINTR is retried, anything else is recorded (the fill runs on worker threads) and
-  // fails the commit; only a true EOF zero-fills, like the reference's ignored short reads (slot.nim:64-65).
-  std::atomic<int> io_errno{0};
-  ChunkFill fill = [fd, offset, &io_errno](uint8_t* dst, uint64_t off, size_t len) {
-    size_t pos = 0;
-    while (pos < len) {
-      const ssize_t got = pread(fd, dst + pos, len - pos, (off_t)(offset + off + pos));
-      if (got < 0) {
-        if (errno == EINTR) continue;
-        int expected = 0;
-        io_errno.compare_exchange_strong(expected, errno);
-        break;
-      }
-      if (got == 0) break;                                                  // EOF: the rest reads as zeros
-      pos += (size_t)got;
-    }
-    if (pos < len) memset(dst + pos, 0, len - pos);
-  };
+  FileSource file;
+  if (!file.open_path(path, offset)) return fail(ctx, CDX_ERR_ARG, "cannot open slot data file `%s`", path);
   SlotSource src;
   src.kind = CDX_SRC_FILE;
-  src.fill = &fill;
+  src.fill = &file.fill;
   rc = commit_from_source(ctx, src, n_bytes, cell_size, block_size, 0, 0, 0, true, true, out);
-  close(fd);
-  if (rc == CDX_OK && io_errno.load() != 0) {
+  if (rc == CDX_OK && file.io_errno.load() != 0) {
     cdx_slot_free(*out);
     *out = nullptr;
-    return fail(ctx, CDX_ERR_ARG, "reading slot data file `%s` failed: %s", path, strerror(io_errno.load()));
+    return fail(ctx, CDX_ERR_ARG, "reading slot data file `%s` failed: %s", path, strerror(file.io_errno.load()));
   }
   return rc;
 }

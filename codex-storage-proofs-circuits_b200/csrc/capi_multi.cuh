@@ -584,36 +584,6 @@ DatasetPlan plan_dataset(const std::vector<uint64_t>& blocks, int n_ranks, size_
   }
   return p;
 }
-
-struct FileSource {      // an open slot data file as a ChunkFill (reads past EOF are zeros: slot.nim:64-65)
-  int fd = -1;
-  uint64_t base = 0;
-  std::atomic<int> io_errno{0};
-  ChunkFill fill;
-  ~FileSource() {
-    if (fd >= 0) close(fd);
-  }
-  bool open_path(const char* path, uint64_t base_offset) {
-    fd = open(path, O_RDONLY);
-    base = base_offset;
-    fill = [this](uint8_t* dst, uint64_t off, size_t len) {
-      size_t pos = 0;
-      while (pos < len) {
-        const ssize_t got = pread(fd, dst + pos, len - pos, (off_t)(base + off + pos));
-        if (got < 0) {
-          if (errno == EINTR) continue;
-          int expected = 0;
-          io_errno.compare_exchange_strong(expected, errno);
-          break;
-        }
-        if (got == 0) break;
-        pos += (size_t)got;
-      }
-      if (pos < len) memset(dst + pos, 0, len - pos);
-    };
-    return fd >= 0;
-  }
-};
 }  // namespace
 
 // bytes of one small slot into a device buffer (batches), queued on st

@@ -576,6 +576,100 @@ def test_cell_sponge_launch_boundary(pkg, ctx, torch_mod):
     small.close()
 
 
+def _tiles(n_blocks, wants):
+    """number of tiles a schedule cuts n_blocks into: `wants` yields each tile's size, the last one is clipped"""
+    done = n = 0
+    for want in wants:
+        if done >= n_blocks:
+            return n
+        done += min(want, n_blocks - done)
+        n += 1
+
+
+def _pinned_wants(n_bytes, block, tile_mib, gradual):
+    n_blocks = n_bytes // block
+    target = tile_mib << 20 if n_bytes >= 1 << 30 else max(n_bytes // 4, 16 << 20)
+    tile = min(max(target // block, 1), n_blocks)
+    if n_blocks > tile and tile >= 8:
+        if gradual:
+            cur = max(tile // 4, 1)
+            while cur < tile:
+                yield cur
+                cur += max(cur // 4, 1)
+        else:
+            yield max(tile // 8, 1)
+            yield tile - max(tile // 8, 1)
+    while True:
+        yield tile
+
+
+def _staged_wants(n_bytes, block, tile_mib):
+    n_blocks = n_bytes // block
+    chunk = max(((tile_mib << 20) // 4) // block, 1)
+    tile = min(4 * chunk, n_blocks)
+    chunk = min(chunk, tile)
+    if n_blocks > tile and tile > chunk:
+        yield chunk
+        yield tile - chunk
+    while True:
+        yield tile
+
+
+def _generated_wants(n_bytes, block, tile_mib):
+    tile = min(max((tile_mib << 20) // block, 1), n_bytes // block)
+    while True:
+        yield tile
+
+
+def test_tile_schedules_of_streamed_sources(pkg, ctx, torch_mod, tmp_path):
+    """the tile schedules of the three streaming pipelines, seen through the launch counter: every tile is one cell-sponge
+    launch (plus one generator launch for generated bytes), so a commit from pinned memory, pageable memory, a file or the
+    fake-data generator launches n_tiles - 1 more kernels than the resident commit of the same bytes, with the same root.
+    Fresh contexts with 16 MiB tiles cover both starts of the pinned pipeline, rings of two and three tiles, and the
+    automatic start, which uses mode 0 on a context's first commit"""
+    import os
+    torch = torch_mod
+    seed, block, cell = 0x5EED, 65536, 2048
+    n_bytes = 4800 * block                                                # 300 MiB
+    d = torch.empty(n_bytes, dtype=torch.uint8, device="cuda")
+    ctx.fake_cells_dev(seed, 0, n_bytes // cell, cell, d.data_ptr())
+    torch.cuda.synchronize()
+    pinned = torch.empty(n_bytes, dtype=torch.uint8, pin_memory=True)
+    pinned.copy_(d)
+    torch.cuda.synchronize()
+    pageable = d.cpu().numpy()
+    path = str(tmp_path / "slot.dat")
+    pageable.tofile(path)
+    n_file, n_fake = _tiles(4800, _staged_wants(n_bytes, block, 16)), _tiles(4800, _generated_wants(n_bytes, block, 16))
+    for ramp, stage_tiles in ((0, 2), (0, 3), (1, 2), (1, 3), (None, None)):
+        env = {"CODEX_COMMIT_TILE_MIB": "16", "CODEX_COMMIT_RAMP": ramp, "CODEX_COMMIT_STAGE_TILES": stage_tiles}
+        saved = {k: os.environ.pop(k, None) for k in env}
+        os.environ.update({k: str(v) for k, v in env.items() if v is not None})
+        try:
+            c = pkg.Context(0)
+        finally:
+            for k, v in saved.items():
+                os.environ.pop(k, None)
+                if v is not None:
+                    os.environ[k] = v
+
+        def delta(commit):
+            before = c.launches
+            with commit() as s:
+                return c.launches - before, s.root
+
+        n_pinned = _tiles(4800, _pinned_wants(n_bytes, block, 16, gradual=ramp == 1))   # automatic start: mode 0 at first
+        got = [delta(lambda: c.slot_commit_host(pinned.data_ptr(), n_bytes=n_bytes)),
+               delta(lambda: c.slot_commit_host(pageable)),
+               delta(lambda: c.slot_commit_file(path, n_bytes)),
+               delta(lambda: c.slot_commit_fake(seed, n_bytes // cell))]
+        resident, root = delta(lambda: c.slot_commit_dev(d.data_ptr(), n_bytes))
+        want = [resident + n_pinned - 1, resident + n_file - 1, resident + n_file - 1, resident + 2 * n_fake - 1]
+        assert [g[0] for g in got] == want, (ramp, stage_tiles)
+        assert all(g[1] == root for g in got), (ramp, stage_tiles)
+        c.close()
+
+
 def test_guard_bands_around_caller_buffers(ctx, torch_mod):
     """device-side memory safety without compute-sanitizer (closed on this pool): every entry point that writes into a
     caller's device buffer is run with ragged sizes (partial warps, partial CTAs, sizes around the launch-width switches)
