@@ -557,6 +557,7 @@ extern "C" int cdx_merkle_layers_host(cdx_ctx* ctx, const uint8_t* leaves, size_
   DevBuf d;
   CU_TRY(ctx, d.alloc(32 * total, ctx->stream));
   CU_TRY(ctx, cudaMemcpyAsync(d.p, leaves, 32 * n, cudaMemcpyHostToDevice, ctx->stream));
+  LAUNCH(ctx, k_canonical_felts, n, ctx->stream, d.u8(), n);       // layer 0 is returned too: leaves >= r come back mod r
   int rc = merkle_layers_on_device(ctx, d.u8(), n, bottom_layer != 0, ctx->stream);
   if (rc) return rc;
   CU_TRY(ctx, cudaMemcpyAsync(layers_out, d.p, 32 * total, cudaMemcpyDeviceToHost, ctx->stream));

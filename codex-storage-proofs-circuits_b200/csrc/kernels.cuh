@@ -234,6 +234,15 @@ __global__ void __launch_bounds__(CDX_BLOCK) k_merkle_level(const uint8_t* __res
   st_felt(out + 32 * i, from_mont(compress_keyed(x, y, key)));
 }
 
+// elements in place to canonical standard form: any 256-bit input is taken mod r.  The bottom layer a caller hands to
+// cdx_merkle_layers_host comes back as layer 0, and outputs are canonical (include/codex_commit.h).
+__global__ void __launch_bounds__(CDX_BLOCK) k_canonical_felts(uint8_t* __restrict__ p, size_t n) {
+  CDX_KERNEL_PROLOGUE();
+  const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  st_felt(p + 32 * i, from_mont(to_mont(ld_felt(p + 32 * i))));
+}
+
 // K3b: one level of MANY Merkle trees at once -- the slot trees of a batch of small slots.  The level-l nodes of all trees
 // are stored tree after tree; in_off / out_off (n_trees + 1 entries each) are the prefix sums of the per-tree widths at
 // the input and the output level.  Per tree the rules are those of k_merkle_level: a trailing single child is paired
