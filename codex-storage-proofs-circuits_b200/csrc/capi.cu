@@ -1022,9 +1022,10 @@ static int hash_cells_host(cdx_ctx* ctx, const uint8_t* data, size_t n_bytes, si
 // so a 100 GiB slot costs 512 MiB of staging.  first_byte is the offset of this range inside its slot.
 static int launch_fake_cells(cdx_ctx* ctx, uint64_t seed, uint64_t first_cell, size_t n_cells, size_t cell_size, void* d_out, cudaStream_t st);
 static int launch_fill_synthetic(cdx_ctx* ctx, uint64_t seed, uint64_t first_word, size_t n_bytes, void* d_out, cudaStream_t st);
+static int fill_synthetic_range(cdx_ctx* ctx, uint64_t seed, uint64_t first_byte, size_t n_bytes, void* d_out, cudaStream_t st);
 static int generate_bytes(cdx_ctx* ctx, uint32_t kind, uint64_t seed, uint64_t first_byte, size_t n_bytes, size_t cell_size, void* d_out, cudaStream_t st) {
   if (kind == CDX_SRC_FAKE) return launch_fake_cells(ctx, seed, first_byte / cell_size, n_bytes / cell_size, cell_size, d_out, st);
-  return launch_fill_synthetic(ctx, seed, first_byte / 8, n_bytes, d_out, st);
+  return fill_synthetic_range(ctx, seed, first_byte, n_bytes, d_out, st);
 }
 static int hash_cells_generated(cdx_ctx* ctx, uint32_t kind, uint64_t seed, uint64_t first_byte, size_t n_bytes, size_t cell_size, size_t block_size,
                                 uint8_t* d_hashes) {
@@ -1449,6 +1450,24 @@ static int launch_fill_synthetic(cdx_ctx* ctx, uint64_t seed, uint64_t first_wor
   const size_t cap = (size_t)ctx->sm_count * 32;
   if (blocks > cap) blocks = cap;
   k_fill_synthetic<<<(unsigned)blocks, 256, 0, st>>>(seed, first_word, n_words, (uint64_t*)d_out);
+  ctx->launches++;
+  CU_TRY(ctx, cudaGetLastError());
+  return CDX_OK;
+}
+
+// Bytes [first_byte, first_byte + n_bytes) of a synthetic slot (include/codex_commit.h, CDX_SRC_SYNTHETIC) into d_out.
+// Whole 8-byte words when the range and the destination allow it, else 4-byte halves: a slot of 100-byte blocks, a tile
+// that starts inside a word, or a batch member behind a 300-byte one.  Cells are multiples of 4 bytes, so every range a
+// slot, a tile or a batch asks for is 4-byte aligned.
+static int fill_synthetic_range(cdx_ctx* ctx, uint64_t seed, uint64_t first_byte, size_t n_bytes, void* d_out, cudaStream_t st) {
+  const uint64_t align = first_byte | n_bytes | (uintptr_t)d_out;
+  if (align % 8 == 0) return launch_fill_synthetic(ctx, seed, first_byte / 8, n_bytes, d_out, st);
+  if (align % 4) return fail(ctx, CDX_ERR_SIZE, "synthetic bytes [%llu,+%zu) are not 4-byte aligned", (unsigned long long)first_byte, n_bytes);
+  const size_t n_halves = n_bytes / 4;
+  size_t blocks = (n_halves + 255) / 256;
+  const size_t cap = (size_t)ctx->sm_count * 32;
+  if (blocks > cap) blocks = cap;
+  k_fill_synthetic_halves<<<(unsigned)blocks, 256, 0, st>>>(seed, first_byte / 4, n_halves, (uint32_t*)d_out);
   ctx->launches++;
   CU_TRY(ctx, cudaGetLastError());
   return CDX_OK;

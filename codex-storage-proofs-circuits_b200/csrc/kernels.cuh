@@ -403,6 +403,18 @@ __global__ void k_fill_synthetic(uint64_t seed, uint64_t first_word, size_t n_wo
   }
 }
 
+// K6c: the same stream in 4-byte halves, for a byte range or a destination that is not 8-byte aligned: half h (h = byte / 4)
+// is the low (h even) or high (h odd) 32 bits of word h / 2, i.e. the bytes of the stream in little-endian order.
+__global__ void k_fill_synthetic_halves(uint64_t seed, uint64_t first_half, size_t n_halves, uint32_t* __restrict__ out) {
+  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n_halves; i += (size_t)gridDim.x * blockDim.x) {
+    const uint64_t h = first_half + i;
+    uint64_t z = seed + (h >> 1) + 0x9e3779b97f4a7c15ull;
+    z = (z ^ (z >> 30)) * 0xbf58476d1ce4e5b9ull;
+    z = (z ^ (z >> 27)) * 0x94d049bb133111ebull;
+    out[i] = (uint32_t)((z ^ (z >> 31)) >> (32 * (h & 1)));
+  }
+}
+
 // Roofline probe: integer multiply streams, ILP 8 per thread, SASS verified (see tools/probes/probe_pipes.cu).
 //   kind 0: IMAD.WIDE.U32 Rd, Ra, Rb, RZ (no carry)   kind 1: IMAD.WIDE.U32.X carry chains of 4 (exactly the
 //   form of the Montgomery rows)   kind 2: 32-bit IMAD

@@ -261,7 +261,9 @@ int cdx_slot_prove_batch_sharded(const cdx_slot* slot, cdx_comm* comm, const uin
 
 typedef enum cdx_source_kind {
   CDX_SRC_FAKE = 0,      /* the reference's fake data: genFakeCell with this seed (nim/slot.nim:23-32) */
-  CDX_SRC_SYNTHETIC = 1, /* counter-based benchmark bytes: word i = splitmix64(seed + i) (cdx_fill_synthetic_dev) */
+  CDX_SRC_SYNTHETIC = 1, /* counter-based benchmark bytes: byte b of the slot is byte b % 8 (little-endian) of
+                            splitmix64(seed + b / 8), for any slot size and any block range or batch offset; where
+                            both are multiples of 8 this is word i = splitmix64(seed + i) (cdx_fill_synthetic_dev) */
   CDX_SRC_FILE = 2,      /* a slot data file, read from offset 0 (nim/dataset.nim:34: <base><k>.dat) */
   CDX_SRC_HOST = 3       /* bytes in host memory */
 } cdx_source_kind;
