@@ -15,6 +15,7 @@ LIB_PATH = os.path.join(_HERE, "libcodexcommit.so")
 
 CDX_OK = 0
 CDX_ERR_ARG, CDX_ERR_SIZE, CDX_ERR_NOT_POW2, CDX_ERR_RANGE, CDX_ERR_CUDA, CDX_ERR_ALLOC, CDX_ERR_STATE = -1, -2, -3, -4, -5, -6, -7
+CDX_ERR_MISMATCH = -8
 
 # every symbol include/codex_commit.h declares: name -> (restype, argtypes)
 _vp, _u8p, _sz, _u64, _u32, _int = C.c_void_p, C.c_char_p, C.c_size_t, C.c_uint64, C.c_uint32, C.c_int
@@ -90,6 +91,9 @@ SYMBOLS = {
     "cdx_dataset_stats": (_int, [_vp, C.POINTER(_u64), C.POINTER(_u32), C.POINTER(_u32), C.POINTER(_u32)]),
     "cdx_dataset_kept_slot": (_vp, [_vp]),
     "cdx_dataset_prove": (_int, [_vp, _vp, _sz, _sz, _vp, _vp, _vp]),
+    "cdx_slot_compact": (_int, [_vp]),
+    "cdx_slot_device_bytes": (_sz, [_vp]),
+    "cdx_slot_prove_from_source": (_int, [_vp, _vp, _vp, _sz, _sz, _sz, _vp, _vp, _vp, _vp]),
     "cdx_group_create": (_int, [C.POINTER(_int), _int, _pp]),
     "cdx_group_destroy": (None, [_vp]),
     "cdx_group_size": (_int, [_vp]),
@@ -540,6 +544,42 @@ class Slot:
         return ([ii[j * n_samples:(j + 1) * n_samples] for j in range(k)],
                 [paths[j * n_samples:(j + 1) * n_samples] for j in range(k)],
                 [leaves[j * n_samples:(j + 1) * n_samples] for j in range(k)])
+
+    def compact(self):
+        """release the block forest below the block hashes (cdx_slot_compact); answer challenges with prove_from_source"""
+        self.ctx._chk(self.ctx.lib.cdx_slot_compact(self.h))
+
+    @property
+    def device_bytes(self) -> int:
+        """device memory the handle holds for its tree levels"""
+        return self.ctx.lib.cdx_slot_device_bytes(self.h)
+
+    def prove_from_source(self, desc, entropies: Sequence[int], n_samples: int, max_depth: int, cells: bool = True):
+        """prove_batch from the slot's bytes, re-hashing only the sampled blocks (works on a compact slot).
+        desc: one (kind, seed | path | buffer, n_bytes) tuple as make_descs takes.
+        -> (indices[k][c], paths[k][c][level], leaves[k][c], cells[k][c] = the cell's bytes, or None with cells=False)"""
+        arr, keep = make_descs([desc])
+        k = len(entropies)
+        total = k * n_samples
+        cell_size = desc[2] // self.shape[0]          # the call fails with CDX_ERR_SIZE before writing if n_bytes is not the slot size
+        ent = b"".join(f2b(e) for e in entropies)
+        idx = (C.c_uint64 * max(total, 1))()
+        out = C.create_string_buffer(32 * total * max_depth if total else 1)
+        leaf = C.create_string_buffer(32 * total if total else 1)
+        cell = C.create_string_buffer(cell_size * total if total else 1) if cells else None
+        self.ctx._chk(self.ctx.lib.cdx_slot_prove_from_source(self.h, arr, _addr(ent), k, n_samples, max_depth, C.addressof(idx), C.addressof(out),
+                                                              C.addressof(leaf), C.addressof(cell) if cells else None))
+        flat = unpack(out.raw[:32 * total * max_depth])
+        leaves = unpack(leaf.raw[:32 * total])
+        ii = list(idx)[:total]
+        paths = [flat[i * max_depth:(i + 1) * max_depth] for i in range(total)]
+        raw = cell.raw if cells else None
+        data = [raw[i * cell_size:(i + 1) * cell_size] if cells else None for i in range(total)]
+        del keep
+        return ([ii[j * n_samples:(j + 1) * n_samples] for j in range(k)],
+                [paths[j * n_samples:(j + 1) * n_samples] for j in range(k)],
+                [leaves[j * n_samples:(j + 1) * n_samples] for j in range(k)],
+                [data[j * n_samples:(j + 1) * n_samples] for j in range(k)])
 
     def export(self) -> bytes:
         n = self.ctx.lib.cdx_slot_export_size(self.h)

@@ -8,6 +8,7 @@
 #include <fcntl.h>
 #include <unistd.h>
 
+#include <algorithm>
 #include <atomic>
 #include <cerrno>
 #include <cstdarg>
@@ -76,6 +77,7 @@ struct cdx_slot {
   uint8_t* d_low = nullptr;     // slot levels 1..top_level (local ranges), concatenated
   uint8_t* d_top = nullptr;     // slot levels top_level..slot_depth (global), concatenated
   bool top0_alias = false;      // top level storage for level top_level aliases forest/low (non-sharded case)
+  bool compact = false;         // cdx_slot_compact: d_forest holds only the block hashes, forest[l < block_depth] are null
   std::vector<uint8_t*> forest, low, top;             // per-level pointers (low[0] aliases forest[block_depth])
   std::vector<uint64_t> low_first, low_count, width;  // width[l] = global width of slot level l
 };
@@ -145,6 +147,7 @@ extern "C" const char* cdx_status_string(int s) {
     case CDX_ERR_CUDA: return "CUDA error / no device";
     case CDX_ERR_ALLOC: return "allocation failed";
     case CDX_ERR_STATE: return "handle is not in the required state";
+    case CDX_ERR_MISMATCH: return "slot bytes do not match the commitment";
     default: return "unknown status";
   }
 }
@@ -609,8 +612,9 @@ static int check_shape(cdx_ctx* ctx, size_t n_bytes, size_t cell_size, size_t bl
 // allocate a slot handle and lay out its layers; on success the caller fills forest[0] and calls build_trees
 // n_local_blocks == 0 is an EMPTY SHARD (a rank that got no chunk of a small slot): it holds nothing below top_level, takes part
 // in the exchange with zero nodes and still gets the replicated top tree; only the sharded entry points create one.
+// compact: a whole slot that keeps only the block hashes of its forest (a compact image being imported).
 static int slot_alloc(cdx_ctx* ctx, uint64_t n_local_blocks, size_t cell_size, size_t block_size, uint64_t first_block,
-                      uint64_t n_total_blocks, int top_level, cudaStream_t st, cdx_slot** out, bool allow_empty = false) {
+                      uint64_t n_total_blocks, int top_level, cudaStream_t st, cdx_slot** out, bool allow_empty = false, bool compact = false) {
   const uint64_t cpb = block_size / cell_size;
   if (n_total_blocks == 0 || (n_local_blocks == 0 && !allow_empty) || first_block + n_local_blocks > n_total_blocks)
     return fail(ctx, CDX_ERR_RANGE, "block range [%llu,+%llu) outside slot of %llu blocks", (unsigned long long)first_block,
@@ -655,8 +659,8 @@ static int slot_alloc(cdx_ctx* ctx, uint64_t n_local_blocks, size_t cell_size, s
   size_t forest_nodes = 0;
   std::vector<size_t> f_off;
   for (uint32_t l = 0; l <= s->block_depth; ++l) {
-    f_off.push_back(forest_nodes);
-    forest_nodes += cpb == 1 ? s->n_local_cells : (s->n_local_cells >> l);
+    f_off.push_back(compact ? 0 : forest_nodes);
+    if (!compact || l == s->block_depth) forest_nodes += cpb == 1 ? s->n_local_cells : (s->n_local_cells >> l);
   }
   // low: slot levels 1..top_level over the local range
   size_t low_nodes = 0;
@@ -678,7 +682,8 @@ static int slot_alloc(cdx_ctx* ctx, uint64_t n_local_blocks, size_t cell_size, s
     cdx_slot_free(s);
     return fail(ctx, CDX_ERR_ALLOC, "cudaMalloc of %zu tree nodes failed: %s", forest_nodes + low_nodes, cudaGetErrorString(e));
   }
-  for (uint32_t l = 0; l <= s->block_depth; ++l) s->forest.push_back(s->d_forest + 32 * f_off[l]);
+  for (uint32_t l = 0; l <= s->block_depth; ++l) s->forest.push_back(compact && l < s->block_depth ? nullptr : s->d_forest + 32 * f_off[l]);
+  s->compact = compact;
   s->low.push_back(s->forest[s->block_depth]);
   for (uint32_t l = 1; l <= s->top_level; ++l) s->low.push_back(s->d_low + 32 * l_off[l]);
   *out = s;
@@ -855,8 +860,9 @@ typedef std::function<int(int t, size_t first, size_t nb, uint8_t* dst, cudaStre
 // Tiles with an even index are produced on `even`, those with an odd index on `odd`; a null stream produces the tile on
 // its compute stream.  Only these streams and ctx->stream2 are ordered after the caller's earlier work on ctx->stream: a
 // copy stream held up for nothing would also hold up upload_table, whose next call waits on the host for the last one.
+// `consume` (may be null) queues more work on a tile, on its compute stream after its sponge, before the buffer is reused.
 static int run_tiles(cdx_ctx* ctx, const std::vector<size_t>& tiles, int n_bufs, cudaStream_t even, cudaStream_t odd, size_t cell_size,
-                     size_t block_size, const TileProducer& produce, uint8_t* d_hashes) {
+                     size_t block_size, const TileProducer& produce, uint8_t* d_hashes, const TileProducer* consume = nullptr) {
   CU_TRY(ctx, cudaEventRecord(ctx->ev_join, ctx->stream));              // d_hashes was allocated on ctx->stream, and
   CU_TRY(ctx, cudaStreamWaitEvent(ctx->stream2, ctx->ev_join, 0));      // earlier work on it may still read the buffers
   if (even) CU_TRY(ctx, cudaStreamWaitEvent(even, ctx->ev_join, 0));
@@ -878,6 +884,10 @@ static int run_tiles(cdx_ctx* ctx, const std::vector<size_t>& tiles, int n_bufs,
     }
     rc = launch_hash_cells(ctx, ctx->d_stage[b], nb * cpb, cell_size, d_hashes + 32 * first * cpb, cs);
     if (rc) return rc;
+    if (consume) {
+      rc = (*consume)(t, first, nb, (uint8_t*)ctx->d_stage[b], cs);
+      if (rc) return rc;
+    }
     CU_TRY(ctx, cudaEventRecord(ctx->ev_consumed[b], cs));
     first += nb;
   }
@@ -948,7 +958,8 @@ static int hash_cells_pinned(cdx_ctx* ctx, const uint8_t* data, size_t n_bytes, 
 // Slot bytes that are not directly DMA-able (a file, or pageable host memory -- what a Nim seq[byte] is).  Host threads
 // fill one of two pinned chunks through `fill(dst, offset, len)` while the copy stream moves the other one into the
 // device tile; a tile is four chunks, copied on the one copy stream into two device buffers.
-static int hash_cells_staged(cdx_ctx* ctx, size_t n_bytes, size_t cell_size, size_t block_size, const ChunkFill& fill, uint8_t* d_hashes) {
+static int hash_cells_staged(cdx_ctx* ctx, size_t n_bytes, size_t cell_size, size_t block_size, const ChunkFill& fill, uint8_t* d_hashes,
+                             const TileProducer* consume = nullptr) {
   const size_t n_blocks = n_bytes / block_size;
   const size_t chunk_bytes_target = (ctx->tile_mib << 20) / 4;              // pinned chunk
   size_t chunk_blocks = chunk_bytes_target / block_size ? chunk_bytes_target / block_size : 1;
@@ -994,7 +1005,8 @@ static int hash_cells_staged(cdx_ctx* ctx, size_t n_bytes, size_t cell_size, siz
     }
     return CDX_OK;
   };
-  rc = run_tiles(ctx, tile_schedule(n_blocks, head, tile_blocks), 2, ctx->copy_stream, ctx->copy_stream, cell_size, block_size, copy, d_hashes);
+  rc = run_tiles(ctx, tile_schedule(n_blocks, head, tile_blocks), 2, ctx->copy_stream, ctx->copy_stream, cell_size, block_size, copy, d_hashes,
+                 consume);
   if (rc) return rc;
   // the pinned chunks are reused by the next call: their last copies must have left the host
   CU_TRY(ctx, cudaEventSynchronize(ctx->ev_h2d[0]));
@@ -1150,14 +1162,17 @@ extern "C" int cdx_slot_commit_fake(cdx_ctx* ctx, uint64_t seed, size_t n_cells,
 }
 
 // ---- persisted commitments ------------------------------------------------------------------------------------
+// A full image ("CDXSLOT1") holds the block forest and slot levels 1..depth; a compact image ("CDXSLOTC", forest_nodes = 0)
+// holds slot levels 0..depth, i.e. the block hashes and everything above them.
 struct SlotImageHeader {
-  char magic[8];              // "CDXSLOT1"
+  char magic[8];              // "CDXSLOT1" or "CDXSLOTC"
   uint64_t cell_size, block_size, n_blocks, forest_nodes, top_nodes;
   uint32_t block_depth, slot_depth;
 };
 
 static size_t forest_node_count(const cdx_slot* s) {
   const uint64_t cpb = s->block_size / s->cell_size;
+  if (s->compact) return s->n_local_blocks;
   size_t n = 0;
   for (uint32_t l = 0; l <= s->block_depth; ++l) n += cpb == 1 ? s->n_local_cells : (s->n_local_cells >> l);
   return n;
@@ -1181,18 +1196,23 @@ extern "C" int cdx_slot_export(const cdx_slot* s, uint8_t* image, size_t image_b
   CU_TRY(ctx, cudaSetDevice(ctx->device));
   SlotImageHeader h;
   memset(&h, 0, sizeof h);
-  memcpy(h.magic, "CDXSLOT1", 8);
+  memcpy(h.magic, s->compact ? "CDXSLOTC" : "CDXSLOT1", 8);
   h.cell_size = s->cell_size;
   h.block_size = s->block_size;
   h.n_blocks = s->n_total_blocks;
-  h.forest_nodes = forest_node_count(s);
+  h.forest_nodes = s->compact ? 0 : forest_node_count(s);
   h.top_nodes = top_node_count(s);
   h.block_depth = s->block_depth;
   h.slot_depth = s->slot_depth;
   memcpy(image, &h, sizeof h);
   uint8_t* p = image + sizeof h;
-  CU_TRY(ctx, cudaMemcpyAsync(p, s->d_forest, 32 * h.forest_nodes, cudaMemcpyDeviceToHost, s->stream));
-  p += 32 * h.forest_nodes;
+  if (s->compact) {
+    CU_TRY(ctx, cudaMemcpyAsync(p, s->top[0], 32 * s->width[0], cudaMemcpyDeviceToHost, s->stream));
+    p += 32 * s->width[0];
+  } else {
+    CU_TRY(ctx, cudaMemcpyAsync(p, s->d_forest, 32 * h.forest_nodes, cudaMemcpyDeviceToHost, s->stream));
+    p += 32 * h.forest_nodes;
+  }
   for (uint32_t l = 1; l <= s->slot_depth; ++l) {
     CU_TRY(ctx, cudaMemcpyAsync(p, s->top[l], 32 * s->width[l], cudaMemcpyDeviceToHost, s->stream));
     p += 32 * s->width[l];
@@ -1207,22 +1227,24 @@ extern "C" int cdx_slot_import(cdx_ctx* ctx, const uint8_t* image, size_t image_
   SlotImageHeader h;
   if (image_bytes < sizeof h) return fail(ctx, CDX_ERR_SIZE, "image too small");
   memcpy(&h, image, sizeof h);
-  if (memcmp(h.magic, "CDXSLOT1", 8) != 0) return fail(ctx, CDX_ERR_ARG, "not a slot image");
+  const bool compact = memcmp(h.magic, "CDXSLOTC", 8) == 0;
+  if (!compact && memcmp(h.magic, "CDXSLOT1", 8) != 0) return fail(ctx, CDX_ERR_ARG, "not a slot image");
   int rc = check_shape(ctx, h.n_blocks * h.block_size, h.cell_size, h.block_size);
   if (rc) return rc;
   CU_TRY(ctx, cudaSetDevice(ctx->device));
   cdx_slot* s = nullptr;
-  rc = slot_alloc(ctx, h.n_blocks, h.cell_size, h.block_size, 0, h.n_blocks, 0, ctx->stream, &s);
+  rc = slot_alloc(ctx, h.n_blocks, h.cell_size, h.block_size, 0, h.n_blocks, 0, ctx->stream, &s, false, compact);
   if (rc) return rc;
   auto body = [&]() -> int {
-    if (forest_node_count(s) != h.forest_nodes || s->block_depth != h.block_depth || s->slot_depth != h.slot_depth)
+    if ((compact ? 0 : forest_node_count(s)) != h.forest_nodes || s->block_depth != h.block_depth || s->slot_depth != h.slot_depth)
       return fail(ctx, CDX_ERR_ARG, "slot image header is inconsistent with its geometry");
     size_t top_nodes = 0;
     for (uint32_t l = 1; l <= s->slot_depth; ++l) top_nodes += s->width[l];
-    if (top_nodes != h.top_nodes || image_bytes != sizeof h + 32 * (h.forest_nodes + h.top_nodes)) return fail(ctx, CDX_ERR_SIZE, "slot image has the wrong length");
+    const size_t level0_nodes = compact ? s->width[0] : h.forest_nodes;   // what precedes slot level 1 in the payload
+    if (top_nodes != h.top_nodes || image_bytes != sizeof h + 32 * (level0_nodes + h.top_nodes)) return fail(ctx, CDX_ERR_SIZE, "slot image has the wrong length");
     const uint8_t* p = image + sizeof h;
-    CU_TRY(ctx, cudaMemcpyAsync(s->d_forest, p, 32 * h.forest_nodes, cudaMemcpyHostToDevice, s->stream));
-    p += 32 * h.forest_nodes;
+    CU_TRY(ctx, cudaMemcpyAsync(s->d_forest, p, 32 * level0_nodes, cudaMemcpyHostToDevice, s->stream));
+    p += 32 * level0_nodes;
     if (top_nodes) CU_TRY(ctx, dev_alloc((void**)&s->d_top, 32 * top_nodes, s->stream));
     s->top.assign(s->slot_depth + 1, nullptr);
     s->top[0] = s->low[0];
@@ -1244,6 +1266,39 @@ extern "C" int cdx_slot_import(cdx_ctx* ctx, const uint8_t* image, size_t image_
   }
   *out = s;
   return CDX_OK;
+}
+
+// Release the block forest below the block hashes (SURVEY.md 8f.2: what a proof server keeps per slot).  Slot level 0 used
+// to alias the end of d_forest; it moves into an allocation of its own, and d_forest is freed on the slot's stream.
+extern "C" int cdx_slot_compact(cdx_slot* s) {
+  if (!s) return CDX_ERR_ARG;
+  cdx_ctx* ctx = s->ctx;
+  if (!exportable(s)) return fail(ctx, CDX_ERR_STATE, "only whole slots with their top tree can be compacted");
+  if (s->compact) return CDX_OK;
+  CU_TRY(ctx, cudaSetDevice(ctx->device));
+  uint8_t* blocks = nullptr;
+  const cudaError_t e = dev_alloc((void**)&blocks, 32 * s->n_local_blocks, s->stream);
+  if (e != cudaSuccess) return fail(ctx, CDX_ERR_ALLOC, "cudaMalloc of %llu block hashes failed: %s", (unsigned long long)s->n_local_blocks, cudaGetErrorString(e));
+  CU_TRY(ctx, cudaMemcpyAsync(blocks, s->forest[s->block_depth], 32 * s->n_local_blocks, cudaMemcpyDeviceToDevice, s->stream));
+  dev_free(s->d_forest, s->stream);
+  s->d_forest = blocks;
+  for (uint32_t l = 0; l < s->block_depth; ++l) s->forest[l] = nullptr;
+  s->forest[s->block_depth] = blocks;
+  s->low[0] = blocks;
+  if (s->top0_alias) s->top[0] = blocks;
+  s->compact = true;
+  CU_TRY(ctx, cudaStreamSynchronize(s->stream));
+  return CDX_OK;
+}
+
+extern "C" size_t cdx_slot_device_bytes(const cdx_slot* s) {
+  if (!s) return 0;
+  size_t nodes = forest_node_count(s);
+  for (uint32_t l = 1; l <= s->top_level; ++l) nodes += s->low_count[l];
+  if (s->has_top)
+    for (uint32_t l = s->top_level; l <= s->slot_depth; ++l)
+      if (!(s->top0_alias && l == s->top_level)) nodes += s->width[l];
+  return 32 * nodes;
 }
 
 extern "C" int cdx_slot_subtree_root_count(const cdx_slot* s, uint64_t* first_node, uint64_t* n_nodes) {
@@ -1305,6 +1360,8 @@ extern "C" int cdx_slot_read_layer(const cdx_slot* s, int tree, uint32_t level, 
   const uint8_t* src = nullptr;
   if (tree == 0) {
     if (level > s->block_depth) return fail(ctx, CDX_ERR_RANGE, "block-forest level %u > %u", level, s->block_depth);
+    if (s->compact && level < s->block_depth)
+      return fail(ctx, CDX_ERR_STATE, "the slot is compact: block-forest level %u was released (cdx_slot_prove_from_source rebuilds sampled blocks)", level);
     const uint64_t cpb = s->block_size / s->cell_size;
     const uint64_t per_block = cpb == 1 ? 1 : (cpb >> level);
     const uint64_t lo = s->first_block * per_block, n = s->n_local_blocks * per_block;
@@ -1471,6 +1528,200 @@ static int fill_synthetic_range(cdx_ctx* ctx, uint64_t seed, uint64_t first_byte
   ctx->launches++;
   CU_TRY(ctx, cudaGetLastError());
   return CDX_OK;
+}
+
+// ---- compact commitments: challenges answered from the slot's bytes ------------------------------------------------
+
+static size_t prove_idx_region(size_t total);   // capi_multi.cuh
+
+// The bytes of the unique sampled blocks ublocks[0..nu) through the tile loop: unique block j lands in its tile at
+// (j - first) * block_size and its cell hashes at d_hashes + 32 * j * cpb.  Generated bytes take one k_generate_blocks launch
+// per tile over the block ids on the device; host memory and files go through the pinned chunks, block by block.
+static int hash_sampled_blocks(cdx_ctx* ctx, const cdx_slot_desc& src, const ChunkFill& file_fill, const std::vector<uint64_t>& ublocks,
+                               const uint64_t* d_ublocks, size_t cell_size, size_t block_size, uint8_t* d_hashes, const TileProducer* consume) {
+  const size_t nu = ublocks.size();
+  if (src.kind == CDX_SRC_FAKE || src.kind == CDX_SRC_SYNTHETIC) {
+    size_t tile_blocks = (ctx->tile_mib << 20) / block_size;
+    if (tile_blocks == 0) tile_blocks = 1;
+    if (tile_blocks > nu) tile_blocks = nu;
+    int rc = ensure_stage(ctx, tile_blocks * block_size);
+    if (rc) return rc;
+    const uint32_t fake = src.kind == CDX_SRC_FAKE ? 1u : 0u;
+    auto generate = [&](int, size_t first, size_t nb, uint8_t* dst, cudaStream_t st) -> int {
+      const size_t units = nb * (fake ? block_size / cell_size : block_size / 4);   // cells or 4-byte halves
+      size_t blocks = (units + 255) / 256;
+      const size_t cap = (size_t)ctx->sm_count * 32;
+      if (blocks > cap) blocks = cap;
+      k_generate_blocks<<<(unsigned)blocks, 256, 0, st>>>(fake, src.seed, d_ublocks + first, nb, (uint64_t)block_size, (uint32_t)cell_size, dst);
+      ctx->launches++;
+      CU_TRY(ctx, cudaGetLastError());
+      return CDX_OK;
+    };
+    return run_tiles(ctx, tile_schedule(nu, {}, tile_blocks), 2, nullptr, nullptr, cell_size, block_size, generate, d_hashes, consume);
+  }
+  const uint8_t* host = src.kind == CDX_SRC_HOST ? src.host : nullptr;
+  ChunkFill fill = [&, host](uint8_t* dst, uint64_t off, size_t len) {   // range offset -> the unique block's bytes in the slot
+    while (len) {
+      const uint64_t j = off / block_size, in = off % block_size;
+      const size_t n = len < block_size - in ? len : (size_t)(block_size - in);
+      const uint64_t at = ublocks[j] * block_size + in;
+      if (host) memcpy(dst, host + at, n);
+      else file_fill(dst, at, n);
+      dst += n;
+      off += n;
+      len -= n;
+    }
+  };
+  return hash_cells_staged(ctx, nu * block_size, cell_size, block_size, fill, d_hashes, consume);
+}
+
+extern "C" int cdx_slot_prove_from_source(const cdx_slot* s, const cdx_slot_desc* source, const uint8_t* entropies, size_t n_challenges,
+                                          size_t n_samples, size_t max_depth, uint64_t* indices_out, uint8_t* paths_out, uint8_t* leaves_out,
+                                          uint8_t* cells_out) {
+  if (!s) return CDX_ERR_ARG;
+  cdx_ctx* ctx = s->ctx;
+  if (!source || !entropies || !indices_out || !paths_out) return fail(ctx, CDX_ERR_ARG, "null pointer");
+  if (!exportable(s)) return fail(ctx, CDX_ERR_STATE, "only whole slots with their top tree can be proven from their bytes");
+  if (n_samples > 0xffffffffu) return fail(ctx, CDX_ERR_SIZE, "too many samples");
+  const size_t cell_size = s->cell_size, block_size = s->block_size, cpb = block_size / cell_size;
+  if (source->n_bytes != s->n_total_blocks * block_size)
+    return fail(ctx, CDX_ERR_SIZE, "the source has %llu bytes, the slot %llu", (unsigned long long)source->n_bytes,
+                (unsigned long long)(s->n_total_blocks * block_size));
+  const uint64_t n_cells_total = s->n_total_blocks << s->cpb_log2;
+  if (max_depth < s->block_depth + s->slot_depth || max_depth > 64)
+    return fail(ctx, CDX_ERR_RANGE, "max_depth %zu < path length %u (padMerkleProof)", max_depth, s->block_depth + s->slot_depth);
+  if (s->block_depth > 32 || s->slot_depth >= 40) return fail(ctx, CDX_ERR_RANGE, "tree too deep for the path plan");
+  const size_t total = n_challenges * n_samples;
+  if (total == 0) return CDX_OK;
+  if (total > (1u << 20)) return fail(ctx, CDX_ERR_SIZE, "too many (challenge, sample) pairs in one call");
+  if (!is_pow2(n_cells_total)) return fail(ctx, CDX_ERR_NOT_POW2, "for this version, `numberOfCells` is assumed to be a power of two");
+  FileSource file;
+  switch (source->kind) {
+    case CDX_SRC_FAKE:
+    case CDX_SRC_SYNTHETIC: break;
+    case CDX_SRC_HOST:
+      if (!source->host) return fail(ctx, CDX_ERR_ARG, "slot descriptor without host pointer");
+      break;
+    case CDX_SRC_FILE:
+      if (!source->path || !file.open_path(source->path, 0))
+        return fail(ctx, CDX_ERR_ARG, "cannot open slot data file `%s`", source->path ? source->path : "(null)");
+      break;
+    default: return fail(ctx, CDX_ERR_ARG, "unknown slot source kind %u", source->kind);
+  }
+  CU_TRY(ctx, cudaSetDevice(ctx->device));
+  if (s->stream != ctx->stream) CU_TRY(ctx, cudaStreamSynchronize(s->stream));   // the retained levels are read on ctx->stream
+  cudaStream_t st = ctx->stream;
+  // [indices 8 B x total, padded to 16 B | paths 32 B x total x max_depth | leaves 32 B x total]: prove_core's layout
+  const size_t idx_bytes = prove_idx_region(total), path_bytes = 32 * total * max_depth, leaf_bytes = 32 * total;
+  DevBuf d_ent, d_all, d_tab, d_forest, d_cells, d_bad;
+  auto body = [&]() -> int {
+    // 1. indices from the retained root, copied back: the one host round trip
+    CU_TRY(ctx, d_all.alloc(idx_bytes + path_bytes + leaf_bytes, st));
+    CU_TRY(ctx, d_ent.alloc(32 * n_challenges, st));
+    CU_TRY(ctx, cudaMemcpyAsync(d_ent.p, entropies, 32 * n_challenges, cudaMemcpyHostToDevice, st));
+    const uint64_t* d_idx = (const uint64_t*)d_all.p;
+    uint8_t* d_paths = d_all.u8() + idx_bytes;
+    uint8_t* d_leaves = d_paths + path_bytes;
+    LAUNCH(ctx, k_cell_indices, total, st, d_ent.u8(), (const uint8_t*)s->top[s->slot_depth], n_cells_total - 1, (uint32_t)n_samples, total,
+           (uint64_t*)d_all.p);
+    CU_TRY(ctx, cudaMemcpyAsync(indices_out, d_idx, 8 * total, cudaMemcpyDeviceToHost, st));
+    CU_TRY(ctx, cudaStreamSynchronize(st));
+    // 2. the sorted unique sampled blocks (duplicate indices are normal, SURVEY.md Appendix C.4: each block is read and
+    // hashed once), each sample's position among them, and the samples in the order of those positions
+    std::vector<uint64_t> ublocks(total);
+    for (size_t i = 0; i < total; ++i) ublocks[i] = indices_out[i] >> s->cpb_log2;
+    std::sort(ublocks.begin(), ublocks.end());
+    ublocks.erase(std::unique(ublocks.begin(), ublocks.end()), ublocks.end());
+    const size_t nu = ublocks.size();
+    std::vector<uint32_t> pos(total), order(total), first_sample(nu + 1, 0);   // samples of unique block j: order[first_sample[j] ..)
+    for (size_t i = 0; i < total; ++i) {
+      pos[i] = (uint32_t)(std::lower_bound(ublocks.begin(), ublocks.end(), indices_out[i] >> s->cpb_log2) - ublocks.begin());
+      ++first_sample[pos[i] + 1];
+    }
+    for (size_t j = 0; j < nu; ++j) first_sample[j + 1] += first_sample[j];
+    {
+      std::vector<uint32_t> next(first_sample.begin(), first_sample.end() - 1);
+      for (size_t i = 0; i < total; ++i) order[next[pos[i]]++] = (uint32_t)i;
+    }
+    std::vector<uint8_t> tab(8 * nu + 8 * total);                               // [unique blocks | pos | order]
+    memcpy(tab.data(), ublocks.data(), 8 * nu);
+    memcpy(tab.data() + 8 * nu, pos.data(), 4 * total);
+    memcpy(tab.data() + 8 * nu + 4 * total, order.data(), 4 * total);
+    int rc = upload_table(ctx, d_tab, tab.data(), tab.size(), st);
+    if (rc) return rc;
+    const uint64_t* d_ublocks = (const uint64_t*)d_tab.p;
+    const uint32_t* d_pos = (const uint32_t*)(d_tab.u8() + 8 * nu);
+    const uint32_t* d_order = d_pos + total;
+    // 3-4. the sampled forest: the unique blocks' cell hashes, then their block trees (build_local_trees' rules)
+    const size_t n_cells = nu * cpb;
+    std::vector<size_t> f_off;
+    size_t forest_nodes = 0;
+    for (uint32_t l = 0; l <= s->block_depth; ++l) {
+      f_off.push_back(forest_nodes);
+      forest_nodes += cpb == 1 ? n_cells : (n_cells >> l);
+    }
+    CU_TRY(ctx, d_forest.alloc(32 * forest_nodes, st));
+    std::vector<uint8_t*> forest;
+    for (uint32_t l = 0; l <= s->block_depth; ++l) forest.push_back(d_forest.u8() + 32 * f_off[l]);
+    if (cells_out) CU_TRY(ctx, d_cells.alloc(cell_size * total, st));
+    // each sample's cell is copied out of its tile while the tile is resident
+    const TileProducer gather = [&](int, size_t first, size_t nb, uint8_t* tile, cudaStream_t cs) -> int {
+      const size_t a = first_sample[first], n = first_sample[first + nb] - a, words = n * (cell_size / 4);
+      if (n == 0) return CDX_OK;
+      size_t blocks = (words + 255) / 256;
+      const size_t cap = (size_t)ctx->sm_count * 32;
+      if (blocks > cap) blocks = cap;
+      k_gather_cells<<<(unsigned)blocks, 256, 0, cs>>>(tile, first, d_order + a, n, d_pos, d_idx, s->cpb_log2, (uint32_t)cell_size,
+                                                        (uint64_t)block_size, d_cells.u8());
+      ctx->launches++;
+      CU_TRY(ctx, cudaGetLastError());
+      return CDX_OK;
+    };
+    rc = hash_sampled_blocks(ctx, *source, file.fill, ublocks, d_ublocks, cell_size, block_size, forest[0], cells_out ? &gather : nullptr);
+    if (rc) return rc;
+    if (cpb == 1) {
+      LAUNCH(ctx, k_merkle_level, n_cells, st, forest[0], n_cells, forest[1], 1u, 1);
+    } else {
+      for (uint32_t l = 0; l < s->block_depth; ++l) {
+        const size_t n = n_cells >> l;
+        LAUNCH(ctx, k_merkle_level, n / 2, st, forest[l], n, forest[l + 1], l == 0 ? 1u : 0u, 0);
+      }
+    }
+    // 5. every recomputed block hash against the retained one
+    CU_TRY(ctx, d_bad.alloc(8, st));
+    CU_TRY(ctx, cudaMemsetAsync(d_bad.p, 0xff, 8, st));
+    LAUNCH(ctx, k_check_sampled_blocks, nu, st, forest[s->block_depth], d_ublocks, nu, (const uint8_t*)s->top[0], (unsigned long long*)d_bad.p);
+    // 6. paths: block levels from the sampled forest, slot levels from the retained tree
+    SampledPathPlan plan;
+    memset(&plan, 0, sizeof plan);
+    for (uint32_t l = 0; l < s->block_depth; ++l) plan.forest[l] = forest[l];
+    for (uint32_t l = 0; l <= s->slot_depth; ++l) {
+      plan.top[l] = s->top[l];
+      plan.width[l] = s->width[l];
+    }
+    plan.block_depth = s->block_depth;
+    plan.slot_depth = s->slot_depth;
+    plan.cells_per_block_log2 = s->cpb_log2;
+    plan.singles = cpb == 1 ? 1u : 0u;
+    const size_t threads = total * (max_depth + 1) * 2;
+    k_gather_paths_sampled<<<grid_for(threads, 256), 256, 0, st>>>(plan, d_idx, d_pos, (uint32_t)total, (uint32_t)max_depth, d_paths, d_leaves);
+    ctx->launches++;
+    CU_TRY(ctx, cudaGetLastError());
+    // 7. one copy back
+    uint64_t bad = 0;
+    CU_TRY(ctx, cudaMemcpyAsync(&bad, d_bad.p, 8, cudaMemcpyDeviceToHost, st));
+    CU_TRY(ctx, cudaMemcpyAsync(paths_out, d_paths, path_bytes, cudaMemcpyDeviceToHost, st));
+    if (leaves_out) CU_TRY(ctx, cudaMemcpyAsync(leaves_out, d_leaves, leaf_bytes, cudaMemcpyDeviceToHost, st));
+    if (cells_out) CU_TRY(ctx, cudaMemcpyAsync(cells_out, d_cells.p, cell_size * total, cudaMemcpyDeviceToHost, st));
+    CU_TRY(ctx, cudaStreamSynchronize(st));
+    if (file.io_errno.load()) return fail(ctx, CDX_ERR_ARG, "reading slot data file `%s` failed: %s", source->path, strerror(file.io_errno.load()));
+    if (bad != UINT64_MAX)
+      return fail(ctx, CDX_ERR_MISMATCH, "bytes of block %llu do not hash to the committed block hash", (unsigned long long)bad);
+    return CDX_OK;
+  };
+  const int rc = body();
+  if (rc) drain_streams(ctx);
+  return rc;
 }
 
 // ---- measurement --------------------------------------------------------------------------------------------

@@ -478,6 +478,7 @@ static size_t prove_idx_region(size_t total) { return (8 * total + 15) & ~(size_
 static int prove_core(const cdx_slot* s, cdx_comm* comm, const uint8_t* entropies, size_t n_challenges, size_t n_samples, const uint64_t* cells,
                       size_t max_depth, bool contribute_indices, uint64_t* indices_out, uint8_t* paths_out, uint8_t* leaves_out) {
   cdx_ctx* ctx = s->ctx;
+  if (s->compact) return fail(ctx, CDX_ERR_STATE, "the slot is compact: its block forest was released, answer challenges with cdx_slot_prove_from_source");
   if (!s->has_top) return fail(ctx, CDX_ERR_STATE, "no top tree yet");
   const uint64_t n_cells_total = s->n_total_blocks << s->cpb_log2;
   if (max_depth < s->block_depth + s->slot_depth || max_depth > 64)

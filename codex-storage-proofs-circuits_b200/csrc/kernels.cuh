@@ -374,13 +374,10 @@ __global__ void k_cell_indices(const uint8_t* __restrict__ entropies, const uint
   out[i] = (((uint64_t)h.l[1] << 32) | h.l[0]) & mask;
 }
 
-// K6a: the reference's fake data, one cell per thread.            slot.nim:23-32, Slot.hs:87-96
-__global__ void k_fake_cells(uint64_t seed, uint64_t first_cell, size_t n_cells, uint32_t cell_size, uint8_t* __restrict__ out) {
-  const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n_cells) return;
-  const uint64_t seed1 = seed + 0xdeadcafeull, seed2 = (first_cell + i) + 0x98765432ull;
+// the reference's fake data for the cell with global index `cell` (cell_size % 4 == 0)
+static __device__ __forceinline__ void fake_cell(uint64_t seed, uint64_t cell, uint32_t cell_size, uint32_t* __restrict__ dst) {
+  const uint64_t seed1 = seed + 0xdeadcafeull, seed2 = cell + 0x98765432ull;
   uint64_t s = 1;
-  uint32_t* dst = reinterpret_cast<uint32_t*>(out + (size_t)cell_size * i);   // cell_size % 4 == 0
   for (uint32_t w = 0; w < cell_size / 4; ++w) {
     uint32_t word = 0;
 #pragma unroll
@@ -393,14 +390,25 @@ __global__ void k_fake_cells(uint64_t seed, uint64_t first_cell, size_t n_cells,
   }
 }
 
+// word w of a synthetic slot seeded with `seed`: splitmix64(seed + w)
+static __device__ __forceinline__ uint64_t synthetic_word(uint64_t seed, uint64_t w) {
+  uint64_t z = seed + w + 0x9e3779b97f4a7c15ull;
+  z = (z ^ (z >> 30)) * 0xbf58476d1ce4e5b9ull;
+  z = (z ^ (z >> 27)) * 0x94d049bb133111ebull;
+  return z ^ (z >> 31);
+}
+
+// K6a: the reference's fake data, one cell per thread.            slot.nim:23-32, Slot.hs:87-96
+__global__ void k_fake_cells(uint64_t seed, uint64_t first_cell, size_t n_cells, uint32_t cell_size, uint8_t* __restrict__ out) {
+  const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n_cells) return;
+  fake_cell(seed, first_cell + i, cell_size, reinterpret_cast<uint32_t*>(out + (size_t)cell_size * i));
+}
+
 // K6b: counter-based synthetic bytes for the large benchmark slots: word i = splitmix64(seed + first_word + i).
 __global__ void k_fill_synthetic(uint64_t seed, uint64_t first_word, size_t n_words, uint64_t* __restrict__ out) {
-  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n_words; i += (size_t)gridDim.x * blockDim.x) {
-    uint64_t z = seed + first_word + i + 0x9e3779b97f4a7c15ull;
-    z = (z ^ (z >> 30)) * 0xbf58476d1ce4e5b9ull;
-    z = (z ^ (z >> 27)) * 0x94d049bb133111ebull;
-    out[i] = z ^ (z >> 31);
-  }
+  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n_words; i += (size_t)gridDim.x * blockDim.x)
+    out[i] = synthetic_word(seed, first_word + i);
 }
 
 // K6c: the same stream in 4-byte halves, for a byte range or a destination that is not 8-byte aligned: half h (h = byte / 4)
@@ -408,10 +416,84 @@ __global__ void k_fill_synthetic(uint64_t seed, uint64_t first_word, size_t n_wo
 __global__ void k_fill_synthetic_halves(uint64_t seed, uint64_t first_half, size_t n_halves, uint32_t* __restrict__ out) {
   for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n_halves; i += (size_t)gridDim.x * blockDim.x) {
     const uint64_t h = first_half + i;
-    uint64_t z = seed + (h >> 1) + 0x9e3779b97f4a7c15ull;
-    z = (z ^ (z >> 30)) * 0xbf58476d1ce4e5b9ull;
-    z = (z ^ (z >> 27)) * 0x94d049bb133111ebull;
-    out[i] = (uint32_t)((z ^ (z >> 31)) >> (32 * (h & 1)));
+    out[i] = (uint32_t)(synthetic_word(seed, h >> 1) >> (32 * (h & 1)));
+  }
+}
+
+// ---- answering challenges from a compact slot (cdx_slot_prove_from_source) --------------------------------------------
+// Only the slot tree is retained; the sampled blocks' bytes are brought back, re-hashed into a "sampled forest" (the
+// block trees of the unique sampled blocks, in ascending block order, laid out like the block forest of a slot made of
+// just those blocks), checked against the retained block hashes, and the paths are gathered from both.
+
+// K6d: generated bytes of a LIST of blocks, back to back: blocks[b] of the slot lands at out + b * block_size.  fake != 0:
+// the reference's fake data, one cell per thread; else the synthetic stream in 4-byte halves (block sizes need not be
+// multiples of 8).  Grid-stride: one launch per tile whatever the number of blocks.
+__global__ void k_generate_blocks(uint32_t fake, uint64_t seed, const uint64_t* __restrict__ blocks, size_t n_blocks, uint64_t block_size,
+                                  uint32_t cell_size, uint8_t* __restrict__ out) {
+  const uint64_t per_block = fake ? block_size / cell_size : block_size / 4;    // cells or halves
+  const size_t n = n_blocks * per_block;
+  for (size_t u = (size_t)blockIdx.x * blockDim.x + threadIdx.x; u < n; u += (size_t)gridDim.x * blockDim.x) {
+    const uint64_t b = u / per_block, k = u % per_block, g = blocks[b] * per_block + k;
+    if (fake) fake_cell(seed, g, cell_size, reinterpret_cast<uint32_t*>(out + (size_t)cell_size * u));
+    else reinterpret_cast<uint32_t*>(out)[u] = (uint32_t)(synthetic_word(seed, g >> 1) >> (32 * (g & 1)));
+  }
+}
+
+// the recomputed hash of sampled block i against the retained slot level 0; bad = the smallest block id that differs
+__global__ void k_check_sampled_blocks(const uint8_t* __restrict__ sampled, const uint64_t* __restrict__ blocks, size_t n,
+                                       const uint8_t* __restrict__ committed, unsigned long long* __restrict__ bad) {
+  const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const uint4* a = reinterpret_cast<const uint4*>(sampled + 32 * i);
+  const uint4* c = reinterpret_cast<const uint4*>(committed + 32 * blocks[i]);
+  const uint4 a0 = a[0], a1 = a[1], c0 = c[0], c1 = c[1];
+  if (a0.x != c0.x || a0.y != c0.y || a0.z != c0.z || a0.w != c0.w || a1.x != c1.x || a1.y != c1.y || a1.z != c1.z || a1.w != c1.w)
+    atomicMin(bad, (unsigned long long)blocks[i]);
+}
+
+struct SampledPathPlan {
+  const uint8_t* forest[32];   // sampled-forest level l, l < block_depth
+  const uint8_t* top[40];      // retained slot-tree level l (all global nodes)
+  uint64_t width[40];          // global width of slot-tree level l
+  uint32_t block_depth, slot_depth, cells_per_block_log2;
+  uint32_t singles;            // one-cell blocks: the block-tree sibling is out of range, i.e. zero (merkle.nim:34)
+};
+
+// K4 for a compact slot: the output of k_gather_paths over the same indices.  pos[s] is the position of sample s's block in
+// the sorted list of unique sampled blocks.  One thread per (sample, level, 16-byte half).
+__global__ void k_gather_paths_sampled(SampledPathPlan plan, const uint64_t* __restrict__ cells, const uint32_t* __restrict__ pos,
+                                       uint32_t n_samples, uint32_t max_depth, uint8_t* __restrict__ out, uint8_t* __restrict__ leaf_out) {
+  const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
+  const uint32_t per_sample = (max_depth + 1) * 2;             // +1: the leaf itself
+  if (t >= n_samples * per_sample) return;
+  const uint32_t s = t / per_sample, rem = t % per_sample, lvl = rem >> 1, half = rem & 1u;
+  const uint64_t cell = cells[s];
+  const uint64_t lc = ((uint64_t)pos[s] << plan.cells_per_block_log2) | (cell & ((1ull << plan.cells_per_block_log2) - 1));   // in the sampled forest
+  uint4 v = make_uint4(0, 0, 0, 0);
+  if (lvl == max_depth) {                                      // leaf slot
+    reinterpret_cast<uint4*>(leaf_out + 32 * (size_t)s)[half] = reinterpret_cast<const uint4*>(plan.forest[0] + 32 * lc)[half];
+    return;
+  }
+  if (lvl < plan.block_depth) {
+    if (!plan.singles) v = reinterpret_cast<const uint4*>(plan.forest[lvl] + 32 * ((lc >> lvl) ^ 1ull))[half];
+  } else if (lvl < plan.block_depth + plan.slot_depth) {
+    const uint32_t l = lvl - plan.block_depth;
+    const uint64_t sib = ((cell >> plan.cells_per_block_log2) >> l) ^ 1ull;
+    if (sib < plan.width[l]) v = reinterpret_cast<const uint4*>(plan.top[l] + 32 * sib)[half];   // out of range -> zero (merkle.nim:34)
+  }
+  reinterpret_cast<uint4*>(out + 32 * ((size_t)s * max_depth + lvl))[half] = v;
+}
+
+// the raw cell of each sample whose block is in the resident tile (tile = unique blocks [first, first + ...)): order[0..n) are
+// those samples, out + s * cell_size receives sample s's cell.  One thread per 4-byte word, grid-stride.
+__global__ void k_gather_cells(const uint8_t* __restrict__ tile, uint64_t first, const uint32_t* __restrict__ order, size_t n,
+                               const uint32_t* __restrict__ pos, const uint64_t* __restrict__ cells, uint32_t cpb_log2, uint32_t cell_size,
+                               uint64_t block_size, uint8_t* __restrict__ out) {
+  const uint32_t words = cell_size / 4;
+  for (size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x; t < n * words; t += (size_t)gridDim.x * blockDim.x) {
+    const uint32_t s = order[t / words], w = (uint32_t)(t % words);
+    const uint8_t* src = tile + (pos[s] - first) * block_size + (cells[s] & ((1ull << cpb_log2) - 1)) * cell_size;
+    reinterpret_cast<uint32_t*>(out + (size_t)cell_size * s)[w] = reinterpret_cast<const uint32_t*>(src)[w];
   }
 }
 

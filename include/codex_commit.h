@@ -38,7 +38,8 @@ typedef enum cdx_status {
   CDX_ERR_RANGE = -4,    /* index out of range (nim/merkle.nim:27) or depth too small (nim/types.nim:29) */
   CDX_ERR_CUDA = -5,     /* CUDA runtime error, or no device */
   CDX_ERR_ALLOC = -6,
-  CDX_ERR_STATE = -7     /* handle not in the state the call needs (e.g. sharded slot without its top tree) */
+  CDX_ERR_STATE = -7,    /* handle not in the state the call needs (e.g. sharded slot without its top tree) */
+  CDX_ERR_MISMATCH = -8  /* slot bytes do not hash to the retained commitment (cdx_slot_prove_from_source) */
 } cdx_status;
 
 typedef struct cdx_ctx cdx_ctx;   /* per-GPU context: device, streams, staging buffers */
@@ -152,7 +153,10 @@ int cdx_slot_set_top_dev(cdx_slot* slot, const void* d_level_nodes, uint64_t n_l
  * commitment instead of re-hashing the slot).  The image is a small header followed by every retained layer (canonical
  * 32-byte elements), about 3.1 % of the slot size; it is self-describing and checked on import.  Only whole
  * (non-sharded, top tree present) slots can be exported.  The reference keeps nothing: it rebuilds the slot tree for
- * every sample (nim/gen_input/bn254.nim:57). */
+ * every sample (nim/gen_input/bn254.nim:57).
+ * A compact slot (cdx_slot_compact) exports a compact image: magic "CDXSLOTC", forest_nodes = 0, slot-tree levels
+ * 0..slot_tree_depth (32 bytes x the sum of their widths, about 0.1 % of the slot at the default geometry); importing it
+ * gives a compact slot. */
 size_t cdx_slot_export_size(const cdx_slot* slot);
 int cdx_slot_export(const cdx_slot* slot, uint8_t* image, size_t image_bytes);
 int cdx_slot_import(cdx_ctx* ctx, const uint8_t* image, size_t image_bytes, cdx_slot** out);
@@ -306,6 +310,36 @@ cdx_slot* cdx_dataset_kept_slot(const cdx_dataset* ds);
  * Replaces: cellIndices + the per-sample proof loop -- nim/sample/bn254.nim:26-27, nim/gen_input/bn254.nim:53-74. */
 int cdx_dataset_prove(const cdx_dataset* ds, const uint8_t entropy[32], size_t n_samples, size_t max_depth, uint64_t* indices_out,
                       uint8_t* paths_out, uint8_t* leaves_out);
+
+/* ---- compact commitments ---------------------------------------------------------------------------------
+ * A challenge samples n_samples cells, and the prover reads those cells' bytes from storage anyway: they are the
+ * `cellData` of the proof input (slotLoadCellData per sample, nim/gen_input/bn254.nim:53-74, nim/slot.nim:51-68).  So a
+ * proof server can keep only the slot tree (the block hashes and above: 32 bytes per block and about as much again for
+ * the levels above, 0.1 % of the slot at 64 KiB blocks) instead of the whole block forest (3.1 %), and rebuild the block
+ * trees of the sampled blocks from their bytes at every challenge.  Doing so also checks that the stored bytes still
+ * hash to the commitment.
+ *
+ * cdx_slot_compact: release the block forest below the block hashes of a whole slot with its top tree (CDX_ERR_STATE for a
+ * shard, a range slot or a slot without its top tree; compacting a compact slot is a no-op).  Afterwards root, shape,
+ * read_layer(tree 1, any level) and read_layer(tree 0, block_tree_depth) work as before; read_layer(tree 0, lower levels),
+ * cdx_slot_cell_paths, cdx_slot_prove_batch and cdx_dataset_prove on a compacted kept slot return CDX_ERR_STATE.
+ * cdx_slot_device_bytes: device memory the handle holds for its tree levels (a diagnostic). */
+int cdx_slot_compact(cdx_slot* slot);
+size_t cdx_slot_device_bytes(const cdx_slot* slot);
+
+/* cdx_slot_prove_batch for a compact or full whole slot, from the slot's bytes: `source` describes them as a dataset slot
+ * does (CDX_SRC_FAKE, CDX_SRC_SYNTHETIC, CDX_SRC_FILE read from offset 0, CDX_SRC_HOST), source->n_bytes must be the slot
+ * size (else CDX_ERR_SIZE).  The cell indices are derived from the retained root; only the unique sampled blocks are read,
+ * hashed into their block trees and checked against the retained block hashes.  indices_out, paths_out and leaves_out
+ * (may be NULL) are byte for byte what cdx_slot_prove_batch gives on the full slot.  cells_out (may be NULL) receives the
+ * raw bytes of every sampled cell, n_challenges x n_samples x cell_size bytes in (challenge, counter) order: the
+ * reference's cellData before elements() (nim/gen_input/bn254.nim:53-74, nim/slot.nim:51-68).  A block whose bytes do
+ * not hash to its retained hash fails the call with CDX_ERR_MISMATCH (the message names the smallest such block; the
+ * outputs are then unspecified); a file that cannot be opened or read is CDX_ERR_ARG, bytes past its end read as zeros.
+ * Limits as cdx_slot_prove_batch.  Returns synchronised. */
+int cdx_slot_prove_from_source(const cdx_slot* slot, const cdx_slot_desc* source, const uint8_t* entropies, size_t n_challenges,
+                               size_t n_samples, size_t max_depth, uint64_t* indices_out, uint8_t* paths_out, uint8_t* leaves_out,
+                               uint8_t* cells_out);
 
 /* ---- all GPUs of one process -------------------------------------------------------------------------------
  * For a single-process host (the Nim cli, the C++ mirror): a group owns one context and one communicator rank per
