@@ -94,6 +94,7 @@ SYMBOLS = {
     "cdx_slot_compact": (_int, [_vp]),
     "cdx_slot_device_bytes": (_sz, [_vp]),
     "cdx_slot_prove_from_source": (_int, [_vp, _vp, _vp, _sz, _sz, _sz, _vp, _vp, _vp, _vp]),
+    "cdx_slots_prove_from_source": (_int, [_vp, _vp, _vp, _sz, _sz, _sz, _vp, _vp, _vp, _vp]),
     "cdx_group_create": (_int, [C.POINTER(_int), _int, _pp]),
     "cdx_group_destroy": (None, [_vp]),
     "cdx_group_size": (_int, [_vp]),
@@ -233,6 +234,29 @@ def _addr(buf) -> int:
     if hasattr(buf, "ctypes"):
         return buf.ctypes.data
     return C.addressof(buf)
+
+
+def _prove_from_source_call(ctx, call, entropies, n_samples, max_depth, cell_size, cells):
+    """runs call(entropies, indices, paths, leaves, cells) of one of the prove_from_source entry points on fresh output
+    buffers -> (indices[k][c], paths[k][c][level], leaves[k][c], cells[k][c] = the cell's bytes, or None with cells=False)"""
+    k = len(entropies)
+    total = k * n_samples
+    ent = b"".join(f2b(e) for e in entropies)
+    idx = (C.c_uint64 * max(total, 1))()
+    out = C.create_string_buffer(32 * total * max_depth if total else 1)
+    leaf = C.create_string_buffer(32 * total if total else 1)
+    cell = C.create_string_buffer(cell_size * total if total else 1) if cells else None
+    ctx._chk(call(_addr(ent), C.addressof(idx), C.addressof(out), C.addressof(leaf), C.addressof(cell) if cells else None))
+    flat = unpack(out.raw[:32 * total * max_depth])
+    leaves = unpack(leaf.raw[:32 * total])
+    ii = list(idx)[:total]
+    paths = [flat[i * max_depth:(i + 1) * max_depth] for i in range(total)]
+    raw = cell.raw if cells else None
+    data = [raw[i * cell_size:(i + 1) * cell_size] if cells else None for i in range(total)]
+    return ([ii[j * n_samples:(j + 1) * n_samples] for j in range(k)],
+            [paths[j * n_samples:(j + 1) * n_samples] for j in range(k)],
+            [leaves[j * n_samples:(j + 1) * n_samples] for j in range(k)],
+            [data[j * n_samples:(j + 1) * n_samples] for j in range(k)])
 
 
 class Context:
@@ -471,6 +495,20 @@ class Context:
     def fill_synthetic_dev(self, seed: int, first_word: int, n_bytes: int, d_out: int, stream: int = 0):
         self._chk(self.lib.cdx_fill_synthetic_dev(self.h, seed & (2**64 - 1), first_word, n_bytes, d_out, stream))
 
+    # ---- compact commitments ----
+    def prove_from_sources(self, rows, n_samples: int, max_depth: int, cells: bool = True):
+        """Slot.prove_from_source over many slots in one call (cdx_slots_prove_from_source).  rows: [(slot, desc, entropy)],
+        desc a (kind, seed | path | buffer, n_bytes) tuple as make_descs takes; a slot may appear in several rows, with
+        equal descriptors.  -> (indices[k][c], paths[k][c][level], leaves[k][c], cells[k][c]), row k answering its own slot"""
+        arr, keep = make_descs([d for _, d, _ in rows])
+        handles = (C.c_void_p * max(len(rows), 1))(*[s.h for s, _, _ in rows])
+        cell_size = rows[0][1][2] // rows[0][0].shape[0] if rows else 0
+        call = lambda ent, idx, out, leaf, cell: self.lib.cdx_slots_prove_from_source(handles, arr, ent, len(rows), n_samples, max_depth,
+                                                                                      idx, out, leaf, cell)
+        res = _prove_from_source_call(self, call, [e for _, _, e in rows], n_samples, max_depth, cell_size, cells)
+        del keep
+        return res
+
     def probe_imad_rate(self, kind: int = 0) -> Tuple[float, float]:
         ops, ms = C.c_double(), C.c_double()
         self._chk(self.lib.cdx_probe_imad_rate(self.h, kind, C.byref(ops), C.byref(ms)))
@@ -559,27 +597,12 @@ class Slot:
         desc: one (kind, seed | path | buffer, n_bytes) tuple as make_descs takes.
         -> (indices[k][c], paths[k][c][level], leaves[k][c], cells[k][c] = the cell's bytes, or None with cells=False)"""
         arr, keep = make_descs([desc])
-        k = len(entropies)
-        total = k * n_samples
         cell_size = desc[2] // self.shape[0]          # the call fails with CDX_ERR_SIZE before writing if n_bytes is not the slot size
-        ent = b"".join(f2b(e) for e in entropies)
-        idx = (C.c_uint64 * max(total, 1))()
-        out = C.create_string_buffer(32 * total * max_depth if total else 1)
-        leaf = C.create_string_buffer(32 * total if total else 1)
-        cell = C.create_string_buffer(cell_size * total if total else 1) if cells else None
-        self.ctx._chk(self.ctx.lib.cdx_slot_prove_from_source(self.h, arr, _addr(ent), k, n_samples, max_depth, C.addressof(idx), C.addressof(out),
-                                                              C.addressof(leaf), C.addressof(cell) if cells else None))
-        flat = unpack(out.raw[:32 * total * max_depth])
-        leaves = unpack(leaf.raw[:32 * total])
-        ii = list(idx)[:total]
-        paths = [flat[i * max_depth:(i + 1) * max_depth] for i in range(total)]
-        raw = cell.raw if cells else None
-        data = [raw[i * cell_size:(i + 1) * cell_size] if cells else None for i in range(total)]
+        call = lambda ent, idx, out, leaf, cell: self.ctx.lib.cdx_slot_prove_from_source(self.h, arr, ent, len(entropies), n_samples, max_depth,
+                                                                                         idx, out, leaf, cell)
+        res = _prove_from_source_call(self.ctx, call, entropies, n_samples, max_depth, cell_size, cells)
         del keep
-        return ([ii[j * n_samples:(j + 1) * n_samples] for j in range(k)],
-                [paths[j * n_samples:(j + 1) * n_samples] for j in range(k)],
-                [leaves[j * n_samples:(j + 1) * n_samples] for j in range(k)],
-                [data[j * n_samples:(j + 1) * n_samples] for j in range(k)])
+        return res
 
     def export(self) -> bytes:
         n = self.ctx.lib.cdx_slot_export_size(self.h)

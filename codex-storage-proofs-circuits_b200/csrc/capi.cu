@@ -16,6 +16,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <functional>
+#include <memory>
 #include <mutex>
 #include <new>
 #include <thread>
@@ -1530,112 +1531,247 @@ static int fill_synthetic_range(cdx_ctx* ctx, uint64_t seed, uint64_t first_byte
   return CDX_OK;
 }
 
-// ---- compact commitments: challenges answered from the slot's bytes ------------------------------------------------
+// ---- compact commitments: challenges answered from the slots' bytes ----------------------------------------------
 
 static size_t prove_idx_region(size_t total);   // capi_multi.cuh
 
-// The bytes of the unique sampled blocks ublocks[0..nu) through the tile loop: unique block j lands in its tile at
-// (j - first) * block_size and its cell hashes at d_hashes + 32 * j * cpb.  Generated bytes take one k_generate_blocks launch
-// per tile over the block ids on the device; host memory and files go through the pinned chunks, block by block.
-static int hash_sampled_blocks(cdx_ctx* ctx, const cdx_slot_desc& src, const ChunkFill& file_fill, const std::vector<uint64_t>& ublocks,
-                               const uint64_t* d_ublocks, size_t cell_size, size_t block_size, uint8_t* d_hashes, const TileProducer* consume) {
-  const size_t nu = ublocks.size();
-  if (src.kind == CDX_SRC_FAKE || src.kind == CDX_SRC_SYNTHETIC) {
+// The sampled forest holds the unique (slot, block) pairs of a call grouped by source class, then by the slot's first row,
+// then by ascending block.  Each class reaches the cell sponge in one pass of the tile loop, whatever its number of slots.
+enum { CLASS_FAKE = 0, CLASS_SYNTHETIC = 1, CLASS_READ = 2, N_CLASSES = 3 };
+
+static uint32_t source_class(uint32_t kind) {
+  return kind == CDX_SRC_FAKE ? CLASS_FAKE : kind == CDX_SRC_SYNTHETIC ? CLASS_SYNTHETIC : CLASS_READ;
+}
+
+// two descriptors of the same bytes: kind, size and the field the kind reads
+static bool same_source(const cdx_slot_desc& a, const cdx_slot_desc& b) {
+  if (a.kind != b.kind || a.n_bytes != b.n_bytes) return false;
+  switch (a.kind) {
+    case CDX_SRC_FAKE:
+    case CDX_SRC_SYNTHETIC: return a.seed == b.seed;
+    case CDX_SRC_FILE: return a.path == b.path || (a.path && b.path && strcmp(a.path, b.path) == 0);
+    case CDX_SRC_HOST: return a.host == b.host;
+    default: return true;                      // refused as an unknown kind
+  }
+}
+
+struct SampledPairs {                          // the sampled forest's pairs, on the host and on the device
+  std::vector<uint64_t> block;                 // pair j: block[j] of slot record slot[j]
+  std::vector<uint32_t> slot;
+  std::vector<const uint8_t*> host;            // per slot record: CDX_SRC_HOST bytes
+  std::vector<const ChunkFill*> file;          // per slot record: CDX_SRC_FILE reader
+  const uint64_t* d_block = nullptr;
+  const uint32_t* d_slot = nullptr;
+  const SampledSlot* d_slots = nullptr;
+};
+
+// The bytes of pairs [begin, begin + n), all of source class cls, through the tile loop: pair j lands in its tile at
+// (j - begin - first) * block_size and its cell hashes at d_hashes + 32 * j * cpb; `consume` sees pair positions.
+// Generated bytes take one k_generate_blocks launch per tile over the pairs on the device; host memory and files go
+// through the pinned chunks, block by block.
+static int hash_sampled_pairs(cdx_ctx* ctx, uint32_t cls, size_t begin, size_t n, const SampledPairs& P, size_t cell_size, size_t block_size,
+                              uint8_t* d_hashes, const TileProducer* consume) {
+  const size_t cpb = block_size / cell_size;
+  uint8_t* hashes = d_hashes + 32 * begin * cpb;
+  const TileProducer shifted = [&](int t, size_t first, size_t nb, uint8_t* tile, cudaStream_t cs) { return (*consume)(t, begin + first, nb, tile, cs); };
+  const TileProducer* hook = consume ? &shifted : nullptr;
+  if (cls != CLASS_READ) {
     size_t tile_blocks = (ctx->tile_mib << 20) / block_size;
     if (tile_blocks == 0) tile_blocks = 1;
-    if (tile_blocks > nu) tile_blocks = nu;
+    if (tile_blocks > n) tile_blocks = n;
     int rc = ensure_stage(ctx, tile_blocks * block_size);
     if (rc) return rc;
-    const uint32_t fake = src.kind == CDX_SRC_FAKE ? 1u : 0u;
+    const uint32_t fake = cls == CLASS_FAKE ? 1u : 0u;
     auto generate = [&](int, size_t first, size_t nb, uint8_t* dst, cudaStream_t st) -> int {
       const size_t units = nb * (fake ? block_size / cell_size : block_size / 4);   // cells or 4-byte halves
       size_t blocks = (units + 255) / 256;
       const size_t cap = (size_t)ctx->sm_count * 32;
       if (blocks > cap) blocks = cap;
-      k_generate_blocks<<<(unsigned)blocks, 256, 0, st>>>(fake, src.seed, d_ublocks + first, nb, (uint64_t)block_size, (uint32_t)cell_size, dst);
+      k_generate_blocks<<<(unsigned)blocks, 256, 0, st>>>(fake, P.d_slots, P.d_slot + begin + first, P.d_block + begin + first, nb,
+                                                          (uint64_t)block_size, (uint32_t)cell_size, dst);
       ctx->launches++;
       CU_TRY(ctx, cudaGetLastError());
       return CDX_OK;
     };
-    return run_tiles(ctx, tile_schedule(nu, {}, tile_blocks), 2, nullptr, nullptr, cell_size, block_size, generate, d_hashes, consume);
+    return run_tiles(ctx, tile_schedule(n, {}, tile_blocks), 2, nullptr, nullptr, cell_size, block_size, generate, hashes, hook);
   }
-  const uint8_t* host = src.kind == CDX_SRC_HOST ? src.host : nullptr;
-  ChunkFill fill = [&, host](uint8_t* dst, uint64_t off, size_t len) {   // range offset -> the unique block's bytes in the slot
+  ChunkFill fill = [&](uint8_t* dst, uint64_t off, size_t len) {   // pass offset -> the pair's bytes in its slot
     while (len) {
-      const uint64_t j = off / block_size, in = off % block_size;
-      const size_t n = len < block_size - in ? len : (size_t)(block_size - in);
-      const uint64_t at = ublocks[j] * block_size + in;
-      if (host) memcpy(dst, host + at, n);
-      else file_fill(dst, at, n);
-      dst += n;
-      off += n;
-      len -= n;
+      const uint64_t j = begin + off / block_size, in = off % block_size;
+      const size_t m = len < block_size - in ? len : (size_t)(block_size - in);
+      const uint64_t at = P.block[j] * block_size + in;
+      const uint32_t r = P.slot[j];
+      if (P.host[r]) memcpy(dst, P.host[r] + at, m);
+      else (*P.file[r])(dst, at, m);
+      dst += m;
+      off += m;
+      len -= m;
     }
   };
-  return hash_cells_staged(ctx, nu * block_size, cell_size, block_size, fill, d_hashes, consume);
+  return hash_cells_staged(ctx, n * block_size, cell_size, block_size, fill, hashes, hook);
 }
 
-extern "C" int cdx_slot_prove_from_source(const cdx_slot* s, const cdx_slot_desc* source, const uint8_t* entropies, size_t n_challenges,
-                                          size_t n_samples, size_t max_depth, uint64_t* indices_out, uint8_t* paths_out, uint8_t* leaves_out,
-                                          uint8_t* cells_out) {
-  if (!s) return CDX_ERR_ARG;
-  cdx_ctx* ctx = s->ctx;
-  if (!source || !entropies || !indices_out || !paths_out) return fail(ctx, CDX_ERR_ARG, "null pointer");
-  if (!exportable(s)) return fail(ctx, CDX_ERR_STATE, "only whole slots with their top tree can be proven from their bytes");
+// cdx_slots_prove_from_source.  one_slot: cdx_slot_prove_from_source, where every row is slots[0] with sources[0] and the
+// messages name no row.
+static int prove_rows(const cdx_slot* const* slots, const cdx_slot_desc* sources, bool one_slot, const uint8_t* entropies, size_t n_rows,
+                      size_t n_samples, size_t max_depth, uint64_t* indices_out, uint8_t* paths_out, uint8_t* leaves_out, uint8_t* cells_out) {
+  cdx_ctx* ctx = slots[0]->ctx;
+  if (!sources || !entropies || !indices_out || !paths_out) return fail(ctx, CDX_ERR_ARG, "null pointer");
+  char pre[48] = "";
+  auto at = [&](size_t row) -> const char* {      // the message prefix naming a row
+    if (!one_slot) snprintf(pre, sizeof pre, "challenge %zu: ", row);
+    return pre;
+  };
+  // the distinct handles in the order of their first rows: slot record r is rec[r], first seen in row first_row[r]
+  std::vector<const cdx_slot*> rec{slots[0]};
+  std::vector<size_t> first_row{0};
+  std::vector<uint32_t> row_slot;
+  if (!one_slot) {
+    row_slot.assign(n_rows, 0);
+    std::unordered_map<const cdx_slot*, uint32_t> seen{{slots[0], 0u}};
+    for (size_t k = 1; k < n_rows; ++k) {
+      if (!slots[k]) return fail(ctx, CDX_ERR_ARG, "%snull slot", at(k));
+      if (slots[k]->ctx != ctx) return fail(ctx, CDX_ERR_ARG, "%sthe slot belongs to another context than challenge 0's", at(k));
+      const auto it = seen.emplace(slots[k], (uint32_t)rec.size());
+      if (it.second) {
+        rec.push_back(slots[k]);
+        first_row.push_back(k);
+      } else if (!same_source(sources[k], sources[first_row[it.first->second]])) {
+        return fail(ctx, CDX_ERR_ARG, "%sthe slot's bytes are described differently in challenge %zu", at(k), first_row[it.first->second]);
+      }
+      row_slot[k] = it.first->second;
+    }
+  }
+  const size_t n_rec = rec.size();
+  auto src_of = [&](size_t r) -> const cdx_slot_desc& { return sources[one_slot ? 0 : first_row[r]]; };
+  for (size_t r = 0; r < n_rec; ++r)
+    if (!exportable(rec[r])) return fail(ctx, CDX_ERR_STATE, "%sonly whole slots with their top tree can be proven from their bytes", at(first_row[r]));
   if (n_samples > 0xffffffffu) return fail(ctx, CDX_ERR_SIZE, "too many samples");
-  const size_t cell_size = s->cell_size, block_size = s->block_size, cpb = block_size / cell_size;
-  if (source->n_bytes != s->n_total_blocks * block_size)
-    return fail(ctx, CDX_ERR_SIZE, "the source has %llu bytes, the slot %llu", (unsigned long long)source->n_bytes,
-                (unsigned long long)(s->n_total_blocks * block_size));
-  const uint64_t n_cells_total = s->n_total_blocks << s->cpb_log2;
-  if (max_depth < s->block_depth + s->slot_depth || max_depth > 64)
-    return fail(ctx, CDX_ERR_RANGE, "max_depth %zu < path length %u (padMerkleProof)", max_depth, s->block_depth + s->slot_depth);
-  if (s->block_depth > 32 || s->slot_depth >= 40) return fail(ctx, CDX_ERR_RANGE, "tree too deep for the path plan");
-  const size_t total = n_challenges * n_samples;
+  const size_t cell_size = rec[0]->cell_size, block_size = rec[0]->block_size, cpb = block_size / cell_size;
+  const uint32_t cpb_log2 = rec[0]->cpb_log2, block_depth = rec[0]->block_depth;
+  uint32_t deepest = 0;
+  for (size_t r = 0; r < n_rec; ++r) {
+    const cdx_slot* s = rec[r];
+    if (s->cell_size != cell_size || s->block_size != block_size)
+      return fail(ctx, CDX_ERR_SIZE, "%sslots of one call share one geometry: cells of %zu and blocks of %zu bytes here, %zu and %zu in challenge 0",
+                  at(first_row[r]), s->cell_size, s->block_size, cell_size, block_size);
+    if (src_of(r).n_bytes != s->n_total_blocks * block_size)
+      return fail(ctx, CDX_ERR_SIZE, "%sthe source has %llu bytes, the slot %llu", at(first_row[r]), (unsigned long long)src_of(r).n_bytes,
+                  (unsigned long long)(s->n_total_blocks * block_size));
+    if (s->slot_depth > rec[deepest]->slot_depth) deepest = (uint32_t)r;
+  }
+  const cdx_slot* ds = rec[deepest];
+  if (max_depth < ds->block_depth + ds->slot_depth || max_depth > 64)
+    return fail(ctx, CDX_ERR_RANGE, "%smax_depth %zu < path length %u (padMerkleProof)", at(first_row[deepest]), max_depth, ds->block_depth + ds->slot_depth);
+  if (ds->block_depth > 32 || ds->slot_depth >= 40) return fail(ctx, CDX_ERR_RANGE, "%stree too deep for the path plan", at(first_row[deepest]));
+  const size_t total = n_rows * n_samples;
   if (total == 0) return CDX_OK;
   if (total > (1u << 20)) return fail(ctx, CDX_ERR_SIZE, "too many (challenge, sample) pairs in one call");
-  if (!is_pow2(n_cells_total)) return fail(ctx, CDX_ERR_NOT_POW2, "for this version, `numberOfCells` is assumed to be a power of two");
-  FileSource file;
-  switch (source->kind) {
-    case CDX_SRC_FAKE:
-    case CDX_SRC_SYNTHETIC: break;
-    case CDX_SRC_HOST:
-      if (!source->host) return fail(ctx, CDX_ERR_ARG, "slot descriptor without host pointer");
-      break;
-    case CDX_SRC_FILE:
-      if (!source->path || !file.open_path(source->path, 0))
-        return fail(ctx, CDX_ERR_ARG, "cannot open slot data file `%s`", source->path ? source->path : "(null)");
-      break;
-    default: return fail(ctx, CDX_ERR_ARG, "unknown slot source kind %u", source->kind);
+  if (one_slot) row_slot.assign(n_rows, 0);
+  for (size_t r = 0; r < n_rec; ++r)
+    if (!is_pow2(rec[r]->n_total_blocks << cpb_log2))
+      return fail(ctx, CDX_ERR_NOT_POW2, "%sfor this version, `numberOfCells` is assumed to be a power of two", at(first_row[r]));
+  // every source readable; files are opened before the pass
+  std::vector<std::unique_ptr<FileSource>> files;
+  SampledPairs P;
+  P.host.assign(n_rec, nullptr);
+  P.file.assign(n_rec, nullptr);
+  std::vector<uint32_t> cls(n_rec);
+  for (size_t r = 0; r < n_rec; ++r) {
+    const cdx_slot_desc& d = src_of(r);
+    switch (d.kind) {
+      case CDX_SRC_FAKE:
+      case CDX_SRC_SYNTHETIC: break;
+      case CDX_SRC_HOST:
+        if (!d.host) return fail(ctx, CDX_ERR_ARG, "%sslot descriptor without host pointer", at(first_row[r]));
+        P.host[r] = d.host;
+        break;
+      case CDX_SRC_FILE:
+        files.emplace_back(new FileSource);
+        if (!d.path || !files.back()->open_path(d.path, 0))
+          return fail(ctx, CDX_ERR_ARG, "%scannot open slot data file `%s`", at(first_row[r]), d.path ? d.path : "(null)");
+        P.file[r] = &files.back()->fill;
+        break;
+      default: return fail(ctx, CDX_ERR_ARG, "%sunknown slot source kind %u", at(first_row[r]), d.kind);
+    }
+    cls[r] = source_class(d.kind);
   }
   CU_TRY(ctx, cudaSetDevice(ctx->device));
-  if (s->stream != ctx->stream) CU_TRY(ctx, cudaStreamSynchronize(s->stream));   // the retained levels are read on ctx->stream
+  {                                                                                 // the retained levels are read on ctx->stream
+    std::vector<cudaStream_t> synced{ctx->stream};
+    for (const cdx_slot* s : rec)
+      if (std::find(synced.begin(), synced.end(), s->stream) == synced.end()) {
+        CU_TRY(ctx, cudaStreamSynchronize(s->stream));
+        synced.push_back(s->stream);
+      }
+  }
   cudaStream_t st = ctx->stream;
   // [indices 8 B x total, padded to 16 B | paths 32 B x total x max_depth | leaves 32 B x total]: prove_core's layout
   const size_t idx_bytes = prove_idx_region(total), path_bytes = 32 * total * max_depth, leaf_bytes = 32 * total;
-  DevBuf d_ent, d_all, d_tab, d_forest, d_cells, d_bad;
+  DevBuf d_rows, d_all, d_tab, d_forest, d_cells, d_bad;
   auto body = [&]() -> int {
-    // 1. indices from the retained root, copied back: the one host round trip
+    // 1. per-row and per-slot tables: [entropies 32 B | root pointer 8 B | mask 8 B per row | slot records | slot levels |
+    // row -> slot record 4 B per row]
+    std::vector<SampledSlot> srec(n_rec);
+    std::vector<SlotLevel> levels;
+    for (size_t r = 0; r < n_rec; ++r) {
+      const cdx_slot* s = rec[r];
+      srec[r].seed = src_of(r).seed;
+      srec[r].first_row = first_row[r];
+      srec[r].levels = (uint32_t)levels.size();
+      srec[r].slot_depth = s->slot_depth;
+      for (uint32_t l = 0; l <= s->slot_depth; ++l) levels.push_back(SlotLevel{s->top[l], s->width[l]});
+    }
+    const size_t o_root = 32 * n_rows, o_mask = o_root + 8 * n_rows, o_slots = o_mask + 8 * n_rows;
+    const size_t o_levels = o_slots + sizeof(SampledSlot) * n_rec, o_row_slot = o_levels + sizeof(SlotLevel) * levels.size();
+    std::vector<uint8_t> rows(o_row_slot + 4 * n_rows);
+    memcpy(rows.data(), entropies, 32 * n_rows);
+    for (size_t k = 0; k < n_rows; ++k) {
+      const cdx_slot* s = rec[row_slot[k]];
+      const uint8_t* root = s->top[s->slot_depth];
+      const uint64_t mask = (s->n_total_blocks << cpb_log2) - 1;
+      memcpy(rows.data() + o_root + 8 * k, &root, 8);
+      memcpy(rows.data() + o_mask + 8 * k, &mask, 8);
+    }
+    memcpy(rows.data() + o_slots, srec.data(), sizeof(SampledSlot) * n_rec);
+    memcpy(rows.data() + o_levels, levels.data(), sizeof(SlotLevel) * levels.size());
+    memcpy(rows.data() + o_row_slot, row_slot.data(), 4 * n_rows);
+    int rc = upload_table(ctx, d_rows, rows.data(), rows.size(), st);
+    if (rc) return rc;
+    P.d_slots = (const SampledSlot*)(d_rows.u8() + o_slots);
+    const SlotLevel* d_levels = (const SlotLevel*)(d_rows.u8() + o_levels);
+    // 2. indices from the retained roots, copied back: the one host round trip
     CU_TRY(ctx, d_all.alloc(idx_bytes + path_bytes + leaf_bytes, st));
-    CU_TRY(ctx, d_ent.alloc(32 * n_challenges, st));
-    CU_TRY(ctx, cudaMemcpyAsync(d_ent.p, entropies, 32 * n_challenges, cudaMemcpyHostToDevice, st));
     const uint64_t* d_idx = (const uint64_t*)d_all.p;
     uint8_t* d_paths = d_all.u8() + idx_bytes;
     uint8_t* d_leaves = d_paths + path_bytes;
-    LAUNCH(ctx, k_cell_indices, total, st, d_ent.u8(), (const uint8_t*)s->top[s->slot_depth], n_cells_total - 1, (uint32_t)n_samples, total,
-           (uint64_t*)d_all.p);
+    LAUNCH(ctx, k_cell_indices_rows, total, st, d_rows.u8(), (const uint8_t* const*)(d_rows.u8() + o_root), (const uint64_t*)(d_rows.u8() + o_mask),
+           (uint32_t)n_samples, total, (uint64_t*)d_all.p);
     CU_TRY(ctx, cudaMemcpyAsync(indices_out, d_idx, 8 * total, cudaMemcpyDeviceToHost, st));
     CU_TRY(ctx, cudaStreamSynchronize(st));
-    // 2. the sorted unique sampled blocks (duplicate indices are normal, SURVEY.md Appendix C.4: each block is read and
-    // hashed once), each sample's position among them, and the samples in the order of those positions
-    std::vector<uint64_t> ublocks(total);
-    for (size_t i = 0; i < total; ++i) ublocks[i] = indices_out[i] >> s->cpb_log2;
-    std::sort(ublocks.begin(), ublocks.end());
-    ublocks.erase(std::unique(ublocks.begin(), ublocks.end()), ublocks.end());
-    const size_t nu = ublocks.size();
-    std::vector<uint32_t> pos(total), order(total), first_sample(nu + 1, 0);   // samples of unique block j: order[first_sample[j] ..)
+    // 3. the sampled forest's unique (slot, block) pairs (duplicate indices are normal, SURVEY.md Appendix C.4: each block is
+    // read and hashed once), each sample's position among them, and the samples in the order of those positions
+    std::vector<std::pair<uint64_t, uint64_t>> key(total), ukey;               // (class << 32 | slot record, block)
     for (size_t i = 0; i < total; ++i) {
-      pos[i] = (uint32_t)(std::lower_bound(ublocks.begin(), ublocks.end(), indices_out[i] >> s->cpb_log2) - ublocks.begin());
+      const uint32_t r = row_slot[i / n_samples];
+      key[i] = {((uint64_t)cls[r] << 32) | r, indices_out[i] >> cpb_log2};
+    }
+    ukey = key;
+    std::sort(ukey.begin(), ukey.end());
+    ukey.erase(std::unique(ukey.begin(), ukey.end()), ukey.end());
+    const size_t nu = ukey.size();
+    P.block.resize(nu);
+    P.slot.resize(nu);
+    size_t class_begin[N_CLASSES + 1] = {0, 0, 0, 0};
+    for (size_t j = 0; j < nu; ++j) {
+      P.block[j] = ukey[j].second;
+      P.slot[j] = (uint32_t)ukey[j].first;
+      ++class_begin[(ukey[j].first >> 32) + 1];
+    }
+    for (int c = 0; c < N_CLASSES; ++c) class_begin[c + 1] += class_begin[c];
+    std::vector<uint32_t> pos(total), order(total), first_sample(nu + 1, 0);   // samples of pair j: order[first_sample[j] ..)
+    for (size_t i = 0; i < total; ++i) {
+      pos[i] = (uint32_t)(std::lower_bound(ukey.begin(), ukey.end(), key[i]) - ukey.begin());
       ++first_sample[pos[i] + 1];
     }
     for (size_t j = 0; j < nu; ++j) first_sample[j + 1] += first_sample[j];
@@ -1643,85 +1779,109 @@ extern "C" int cdx_slot_prove_from_source(const cdx_slot* s, const cdx_slot_desc
       std::vector<uint32_t> next(first_sample.begin(), first_sample.end() - 1);
       for (size_t i = 0; i < total; ++i) order[next[pos[i]]++] = (uint32_t)i;
     }
-    std::vector<uint8_t> tab(8 * nu + 8 * total);                               // [unique blocks | pos | order]
-    memcpy(tab.data(), ublocks.data(), 8 * nu);
+    std::vector<uint8_t> tab(8 * nu + 8 * total + 4 * nu);                     // [pair blocks | pos | order | pair slot records]
+    memcpy(tab.data(), P.block.data(), 8 * nu);
     memcpy(tab.data() + 8 * nu, pos.data(), 4 * total);
     memcpy(tab.data() + 8 * nu + 4 * total, order.data(), 4 * total);
-    int rc = upload_table(ctx, d_tab, tab.data(), tab.size(), st);
+    memcpy(tab.data() + 8 * nu + 8 * total, P.slot.data(), 4 * nu);
+    rc = upload_table(ctx, d_tab, tab.data(), tab.size(), st);
     if (rc) return rc;
-    const uint64_t* d_ublocks = (const uint64_t*)d_tab.p;
+    P.d_block = (const uint64_t*)d_tab.p;
     const uint32_t* d_pos = (const uint32_t*)(d_tab.u8() + 8 * nu);
     const uint32_t* d_order = d_pos + total;
-    // 3-4. the sampled forest: the unique blocks' cell hashes, then their block trees (build_local_trees' rules)
+    P.d_slot = d_order + total;
+    // 4-5. the sampled forest: the pairs' cell hashes, one tile pass per source class, then their block trees
+    // (build_local_trees' rules)
     const size_t n_cells = nu * cpb;
     std::vector<size_t> f_off;
     size_t forest_nodes = 0;
-    for (uint32_t l = 0; l <= s->block_depth; ++l) {
+    for (uint32_t l = 0; l <= block_depth; ++l) {
       f_off.push_back(forest_nodes);
       forest_nodes += cpb == 1 ? n_cells : (n_cells >> l);
     }
     CU_TRY(ctx, d_forest.alloc(32 * forest_nodes, st));
     std::vector<uint8_t*> forest;
-    for (uint32_t l = 0; l <= s->block_depth; ++l) forest.push_back(d_forest.u8() + 32 * f_off[l]);
+    for (uint32_t l = 0; l <= block_depth; ++l) forest.push_back(d_forest.u8() + 32 * f_off[l]);
     if (cells_out) CU_TRY(ctx, d_cells.alloc(cell_size * total, st));
-    // each sample's cell is copied out of its tile while the tile is resident
+    // each sample's cell is copied out of its tile while the tile is resident (first: the tile's first pair)
     const TileProducer gather = [&](int, size_t first, size_t nb, uint8_t* tile, cudaStream_t cs) -> int {
       const size_t a = first_sample[first], n = first_sample[first + nb] - a, words = n * (cell_size / 4);
       if (n == 0) return CDX_OK;
       size_t blocks = (words + 255) / 256;
       const size_t cap = (size_t)ctx->sm_count * 32;
       if (blocks > cap) blocks = cap;
-      k_gather_cells<<<(unsigned)blocks, 256, 0, cs>>>(tile, first, d_order + a, n, d_pos, d_idx, s->cpb_log2, (uint32_t)cell_size,
+      k_gather_cells<<<(unsigned)blocks, 256, 0, cs>>>(tile, first, d_order + a, n, d_pos, d_idx, cpb_log2, (uint32_t)cell_size,
                                                         (uint64_t)block_size, d_cells.u8());
       ctx->launches++;
       CU_TRY(ctx, cudaGetLastError());
       return CDX_OK;
     };
-    rc = hash_sampled_blocks(ctx, *source, file.fill, ublocks, d_ublocks, cell_size, block_size, forest[0], cells_out ? &gather : nullptr);
-    if (rc) return rc;
+    for (uint32_t c = 0; c < N_CLASSES; ++c) {
+      if (class_begin[c + 1] == class_begin[c]) continue;
+      rc = hash_sampled_pairs(ctx, c, class_begin[c], class_begin[c + 1] - class_begin[c], P, cell_size, block_size, forest[0],
+                              cells_out ? &gather : nullptr);
+      if (rc) return rc;
+    }
     if (cpb == 1) {
       LAUNCH(ctx, k_merkle_level, n_cells, st, forest[0], n_cells, forest[1], 1u, 1);
     } else {
-      for (uint32_t l = 0; l < s->block_depth; ++l) {
+      for (uint32_t l = 0; l < block_depth; ++l) {
         const size_t n = n_cells >> l;
         LAUNCH(ctx, k_merkle_level, n / 2, st, forest[l], n, forest[l + 1], l == 0 ? 1u : 0u, 0);
       }
     }
-    // 5. every recomputed block hash against the retained one
+    // 6. every recomputed block hash against its slot's retained one
     CU_TRY(ctx, d_bad.alloc(8, st));
     CU_TRY(ctx, cudaMemsetAsync(d_bad.p, 0xff, 8, st));
-    LAUNCH(ctx, k_check_sampled_blocks, nu, st, forest[s->block_depth], d_ublocks, nu, (const uint8_t*)s->top[0], (unsigned long long*)d_bad.p);
-    // 6. paths: block levels from the sampled forest, slot levels from the retained tree
+    LAUNCH(ctx, k_check_sampled_blocks, nu, st, forest[block_depth], P.d_block, P.d_slot, nu, P.d_slots, d_levels, (unsigned long long*)d_bad.p);
+    // 7. paths: block levels from the sampled forest, slot levels from each row's slot record
     SampledPathPlan plan;
     memset(&plan, 0, sizeof plan);
-    for (uint32_t l = 0; l < s->block_depth; ++l) plan.forest[l] = forest[l];
-    for (uint32_t l = 0; l <= s->slot_depth; ++l) {
-      plan.top[l] = s->top[l];
-      plan.width[l] = s->width[l];
-    }
-    plan.block_depth = s->block_depth;
-    plan.slot_depth = s->slot_depth;
-    plan.cells_per_block_log2 = s->cpb_log2;
+    for (uint32_t l = 0; l < block_depth; ++l) plan.forest[l] = forest[l];
+    plan.row_slot = (const uint32_t*)(d_rows.u8() + o_row_slot);
+    plan.slots = P.d_slots;
+    plan.levels = d_levels;
+    plan.block_depth = block_depth;
+    plan.cells_per_block_log2 = cpb_log2;
+    plan.n_samples = (uint32_t)n_samples;
     plan.singles = cpb == 1 ? 1u : 0u;
     const size_t threads = total * (max_depth + 1) * 2;
     k_gather_paths_sampled<<<grid_for(threads, 256), 256, 0, st>>>(plan, d_idx, d_pos, (uint32_t)total, (uint32_t)max_depth, d_paths, d_leaves);
     ctx->launches++;
     CU_TRY(ctx, cudaGetLastError());
-    // 7. one copy back
+    // 8. one copy back
     uint64_t bad = 0;
     CU_TRY(ctx, cudaMemcpyAsync(&bad, d_bad.p, 8, cudaMemcpyDeviceToHost, st));
     CU_TRY(ctx, cudaMemcpyAsync(paths_out, d_paths, path_bytes, cudaMemcpyDeviceToHost, st));
     if (leaves_out) CU_TRY(ctx, cudaMemcpyAsync(leaves_out, d_leaves, leaf_bytes, cudaMemcpyDeviceToHost, st));
     if (cells_out) CU_TRY(ctx, cudaMemcpyAsync(cells_out, d_cells.p, cell_size * total, cudaMemcpyDeviceToHost, st));
     CU_TRY(ctx, cudaStreamSynchronize(st));
-    if (file.io_errno.load()) return fail(ctx, CDX_ERR_ARG, "reading slot data file `%s` failed: %s", source->path, strerror(file.io_errno.load()));
+    for (size_t r = 0, f = 0; r < n_rec; ++r)
+      if (P.file[r] && files[f++]->io_errno.load())
+        return fail(ctx, CDX_ERR_ARG, "%sreading slot data file `%s` failed: %s", at(first_row[r]), src_of(r).path, strerror(files[f - 1]->io_errno.load()));
     if (bad != UINT64_MAX)
-      return fail(ctx, CDX_ERR_MISMATCH, "bytes of block %llu do not hash to the committed block hash", (unsigned long long)bad);
+      return fail(ctx, CDX_ERR_MISMATCH, "%sbytes of block %llu do not hash to the committed block hash", at(bad >> 44),
+                  (unsigned long long)(bad & ((1ull << 44) - 1)));
     return CDX_OK;
   };
   const int rc = body();
   if (rc) drain_streams(ctx);
   return rc;
+}
+
+extern "C" int cdx_slot_prove_from_source(const cdx_slot* s, const cdx_slot_desc* source, const uint8_t* entropies, size_t n_challenges,
+                                          size_t n_samples, size_t max_depth, uint64_t* indices_out, uint8_t* paths_out, uint8_t* leaves_out,
+                                          uint8_t* cells_out) {
+  if (!s) return CDX_ERR_ARG;
+  return prove_rows(&s, source, true, entropies, n_challenges, n_samples, max_depth, indices_out, paths_out, leaves_out, cells_out);
+}
+
+extern "C" int cdx_slots_prove_from_source(const cdx_slot* const* slots, const cdx_slot_desc* sources, const uint8_t* entropies,
+                                           size_t n_challenges, size_t n_samples, size_t max_depth, uint64_t* indices_out, uint8_t* paths_out,
+                                           uint8_t* leaves_out, uint8_t* cells_out) {
+  if (n_challenges == 0) return CDX_OK;
+  if (!slots || !slots[0]) return CDX_ERR_ARG;
+  return prove_rows(slots, sources, false, entropies, n_challenges, n_samples, max_depth, indices_out, paths_out, leaves_out, cells_out);
 }
 
 // ---- measurement --------------------------------------------------------------------------------------------

@@ -356,22 +356,36 @@ __global__ void __launch_bounds__(CDX_BLOCK) k_reconstruct_roots(const uint8_t* 
 
 // K5: sampled cell indices, one thread per (challenge, counter).   sample/bn254.nim:16-27, types/bn254.nim:47-59
 // entropies: n_challenges x 32 B, root: 32 B (both canonical), out[ch * n_samples + c-1].
-__global__ void k_cell_indices(const uint8_t* __restrict__ entropies, const uint8_t* __restrict__ root, uint64_t mask, uint32_t n_samples,
-                               size_t total, uint64_t* __restrict__ out) {
-  CDX_KERNEL_PROLOGUE();
-  const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= total) return;
-  const size_t ch = i / n_samples;
-  const uint32_t counter = (uint32_t)(i % n_samples) + 1u;     // counters run 1..nSamples
+static __device__ __forceinline__ uint64_t cell_index(const uint8_t* entropy, const uint8_t* root, uint32_t counter, uint64_t mask) {
   auto get = [&](uint32_t k) {
-    if (k == 0) return ld_felt(entropies + 32 * ch);
+    if (k == 0) return ld_felt(entropy);
     if (k == 1) return ld_felt(root);
     Fr c = fr_zero();
     c.l[0] = counter;
     return c;
   };
   Fr h = from_mont(sponge_elems(get, 3, 2));
-  out[i] = (((uint64_t)h.l[1] << 32) | h.l[0]) & mask;
+  return (((uint64_t)h.l[1] << 32) | h.l[0]) & mask;
+}
+
+__global__ void k_cell_indices(const uint8_t* __restrict__ entropies, const uint8_t* __restrict__ root, uint64_t mask, uint32_t n_samples,
+                               size_t total, uint64_t* __restrict__ out) {
+  CDX_KERNEL_PROLOGUE();
+  const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= total) return;
+  const size_t ch = i / n_samples;
+  out[i] = cell_index(entropies + 32 * ch, root, (uint32_t)(i % n_samples) + 1u, mask);   // counters run 1..nSamples
+}
+
+// K5b: the same over challenges against different slots: challenge ch samples the slot whose root is roots[ch] and whose
+// cell count is masks[ch] + 1.
+__global__ void k_cell_indices_rows(const uint8_t* __restrict__ entropies, const uint8_t* const* __restrict__ roots,
+                                    const uint64_t* __restrict__ masks, uint32_t n_samples, size_t total, uint64_t* __restrict__ out) {
+  CDX_KERNEL_PROLOGUE();
+  const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= total) return;
+  const size_t ch = i / n_samples;
+  out[i] = cell_index(entropies + 32 * ch, roots[ch], (uint32_t)(i % n_samples) + 1u, masks[ch]);
 }
 
 // the reference's fake data for the cell with global index `cell` (cell_size % 4 == 0)
@@ -420,47 +434,67 @@ __global__ void k_fill_synthetic_halves(uint64_t seed, uint64_t first_half, size
   }
 }
 
-// ---- answering challenges from a compact slot (cdx_slot_prove_from_source) --------------------------------------------
-// Only the slot tree is retained; the sampled blocks' bytes are brought back, re-hashed into a "sampled forest" (the
-// block trees of the unique sampled blocks, in ascending block order, laid out like the block forest of a slot made of
-// just those blocks), checked against the retained block hashes, and the paths are gathered from both.
+// ---- answering challenges from compact slots (cdx_slots_prove_from_source) ----------------------------------------------
+// Only the slot trees are retained; the sampled blocks' bytes are brought back, re-hashed into a "sampled forest" (the
+// block trees of the unique sampled (slot, block) pairs, laid out like the block forest of a slot made of just those
+// blocks), checked against the retained block hashes, and the paths are gathered from both.  Every slot of one call has
+// the same geometry, so the pairs of all slots share the forest's levels.
 
-// K6d: generated bytes of a LIST of blocks, back to back: blocks[b] of the slot lands at out + b * block_size.  fake != 0:
-// the reference's fake data, one cell per thread; else the synthetic stream in 4-byte halves (block sizes need not be
-// multiples of 8).  Grid-stride: one launch per tile whatever the number of blocks.
-__global__ void k_generate_blocks(uint32_t fake, uint64_t seed, const uint64_t* __restrict__ blocks, size_t n_blocks, uint64_t block_size,
-                                  uint32_t cell_size, uint8_t* __restrict__ out) {
+struct SlotLevel {             // one retained slot-tree level: all global nodes of it
+  const uint8_t* nodes;
+  uint64_t width;
+};
+
+struct SampledSlot {           // one distinct slot of the call, in the order of its first challenge row
+  uint64_t seed;               // generated sources: the slot's seed
+  uint64_t first_row;          // its first challenge row (the mismatch key)
+  uint32_t levels;             // its slot level 0 in the level table; levels .. levels + slot_depth
+  uint32_t slot_depth;
+};
+
+// K6d: generated bytes of a LIST of (slot, block) pairs, back to back: block blocks[b] of slot slot_of[b] lands at
+// out + b * block_size.  fake != 0: the reference's fake data, one cell per thread; else the synthetic stream in 4-byte
+// halves (block sizes need not be multiples of 8).  Grid-stride: one launch per tile whatever the number of blocks.
+__global__ void k_generate_blocks(uint32_t fake, const SampledSlot* __restrict__ slots, const uint32_t* __restrict__ slot_of,
+                                  const uint64_t* __restrict__ blocks, size_t n_blocks, uint64_t block_size, uint32_t cell_size,
+                                  uint8_t* __restrict__ out) {
   const uint64_t per_block = fake ? block_size / cell_size : block_size / 4;    // cells or halves
   const size_t n = n_blocks * per_block;
   for (size_t u = (size_t)blockIdx.x * blockDim.x + threadIdx.x; u < n; u += (size_t)gridDim.x * blockDim.x) {
     const uint64_t b = u / per_block, k = u % per_block, g = blocks[b] * per_block + k;
+    const uint64_t seed = slots[slot_of[b]].seed;
     if (fake) fake_cell(seed, g, cell_size, reinterpret_cast<uint32_t*>(out + (size_t)cell_size * u));
     else reinterpret_cast<uint32_t*>(out)[u] = (uint32_t)(synthetic_word(seed, g >> 1) >> (32 * (g & 1)));
   }
 }
 
-// the recomputed hash of sampled block i against the retained slot level 0; bad = the smallest block id that differs
-__global__ void k_check_sampled_blocks(const uint8_t* __restrict__ sampled, const uint64_t* __restrict__ blocks, size_t n,
-                                       const uint8_t* __restrict__ committed, unsigned long long* __restrict__ bad) {
+// the recomputed hash of sampled pair i against its slot's retained level 0; bad = the smallest key (slot's first row << 44
+// | block) among the pairs that differ
+__global__ void k_check_sampled_blocks(const uint8_t* __restrict__ sampled, const uint64_t* __restrict__ blocks,
+                                       const uint32_t* __restrict__ slot_of, size_t n, const SampledSlot* __restrict__ slots,
+                                       const SlotLevel* __restrict__ levels, unsigned long long* __restrict__ bad) {
   const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
+  const SampledSlot& sl = slots[slot_of[i]];
   const uint4* a = reinterpret_cast<const uint4*>(sampled + 32 * i);
-  const uint4* c = reinterpret_cast<const uint4*>(committed + 32 * blocks[i]);
+  const uint4* c = reinterpret_cast<const uint4*>(levels[sl.levels].nodes + 32 * blocks[i]);
   const uint4 a0 = a[0], a1 = a[1], c0 = c[0], c1 = c[1];
   if (a0.x != c0.x || a0.y != c0.y || a0.z != c0.z || a0.w != c0.w || a1.x != c1.x || a1.y != c1.y || a1.z != c1.z || a1.w != c1.w)
-    atomicMin(bad, (unsigned long long)blocks[i]);
+    atomicMin(bad, (unsigned long long)((sl.first_row << 44) | blocks[i]));
 }
 
 struct SampledPathPlan {
   const uint8_t* forest[32];   // sampled-forest level l, l < block_depth
-  const uint8_t* top[40];      // retained slot-tree level l (all global nodes)
-  uint64_t width[40];          // global width of slot-tree level l
-  uint32_t block_depth, slot_depth, cells_per_block_log2;
+  const uint32_t* row_slot;    // challenge row -> its slot record
+  const SampledSlot* slots;
+  const SlotLevel* levels;
+  uint32_t block_depth, cells_per_block_log2, n_samples;
   uint32_t singles;            // one-cell blocks: the block-tree sibling is out of range, i.e. zero (merkle.nim:34)
 };
 
-// K4 for a compact slot: the output of k_gather_paths over the same indices.  pos[s] is the position of sample s's block in
-// the sorted list of unique sampled blocks.  One thread per (sample, level, 16-byte half).
+// K4 for compact slots: per row, the output of k_gather_paths on that row's slot over the same indices.  pos[s] is the
+// position of sample s's (slot, block) pair in the sampled forest; sample s belongs to row s / n_samples.  A slot shallower
+// than max_depth gets zeros above its slot depth.  One thread per (sample, level, 16-byte half).
 __global__ void k_gather_paths_sampled(SampledPathPlan plan, const uint64_t* __restrict__ cells, const uint32_t* __restrict__ pos,
                                        uint32_t n_samples, uint32_t max_depth, uint8_t* __restrict__ out, uint8_t* __restrict__ leaf_out) {
   const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
@@ -476,10 +510,14 @@ __global__ void k_gather_paths_sampled(SampledPathPlan plan, const uint64_t* __r
   }
   if (lvl < plan.block_depth) {
     if (!plan.singles) v = reinterpret_cast<const uint4*>(plan.forest[lvl] + 32 * ((lc >> lvl) ^ 1ull))[half];
-  } else if (lvl < plan.block_depth + plan.slot_depth) {
+  } else {
+    const SampledSlot& sl = plan.slots[plan.row_slot[s / plan.n_samples]];
     const uint32_t l = lvl - plan.block_depth;
-    const uint64_t sib = ((cell >> plan.cells_per_block_log2) >> l) ^ 1ull;
-    if (sib < plan.width[l]) v = reinterpret_cast<const uint4*>(plan.top[l] + 32 * sib)[half];   // out of range -> zero (merkle.nim:34)
+    if (l < sl.slot_depth) {
+      const SlotLevel lv = plan.levels[sl.levels + l];
+      const uint64_t sib = ((cell >> plan.cells_per_block_log2) >> l) ^ 1ull;
+      if (sib < lv.width) v = reinterpret_cast<const uint4*>(lv.nodes + 32 * sib)[half];   // out of range -> zero (merkle.nim:34)
+    }
   }
   reinterpret_cast<uint4*>(out + 32 * ((size_t)s * max_depth + lvl))[half] = v;
 }

@@ -341,6 +341,28 @@ int cdx_slot_prove_from_source(const cdx_slot* slot, const cdx_slot_desc* source
                                size_t n_samples, size_t max_depth, uint64_t* indices_out, uint8_t* paths_out, uint8_t* leaves_out,
                                uint8_t* cells_out);
 
+/* cdx_slot_prove_from_source for many slots at once.  Challenge k is entropies + 32 k against slots[k], whose bytes
+ * sources[k] describes (as for cdx_slot_prove_from_source).  A handle may appear in several rows; those rows must give equal
+ * descriptors (kind, seed / path / host pointer, n_bytes), and each of its sampled blocks is read and hashed once for all of them.
+ * Outputs use the layout of cdx_slot_prove_from_source with n_challenges rows: indices_out[k * n_samples + c - 1], paths_out,
+ * leaves_out, cells_out (the last three may be NULL).  Row k is byte for byte what cdx_slot_prove_batch(slots[k], entropy k)
+ * gives on the full slot.  A shallower slot's paths are zero-padded to max_depth.
+ * A proof server gathers one period's challenges over all its slots into one call: the sampled blocks of every slot reach
+ * the cell sponge together (one tile pass per source class: fake data, synthetic bytes, host memory and files), so the
+ * call costs about what one slot with that many challenges costs, not the single-challenge latency once per slot.
+ * n_challenges == 0 is CDX_OK and touches nothing.  CDX_ERR_ARG: a null slots, sources, entropies, indices_out or paths_out,
+ * slots of different contexts, one handle with differing descriptors, a file that cannot be opened or read (bytes past
+ * its end read as zeros).  CDX_ERR_SIZE: slots whose cell_size or block_size differ, sources[k].n_bytes not the slot's
+ * size, more than 2^20 (challenge, sample) pairs.  CDX_ERR_STATE: a range slot, a shard or a slot without its top tree.
+ * CDX_ERR_NOT_POW2: a slot whose cell count is not a power of two.  CDX_ERR_RANGE: max_depth below the deepest slot's path
+ * length or above 64.  Compact and full slots may be mixed.  CDX_ERR_MISMATCH: a sampled block does not hash to its
+ * retained hash; the message reads "challenge k: bytes of block N do not hash to the committed block hash", naming, among
+ * the slots with a bad block, the one whose first row comes first: k is that row and N its smallest bad block (the
+ * outputs are then unspecified).  Returns synchronised. */
+int cdx_slots_prove_from_source(const cdx_slot* const* slots, const cdx_slot_desc* sources, const uint8_t* entropies,
+                                size_t n_challenges, size_t n_samples, size_t max_depth, uint64_t* indices_out,
+                                uint8_t* paths_out, uint8_t* leaves_out, uint8_t* cells_out);
+
 /* ---- all GPUs of one process -------------------------------------------------------------------------------
  * For a single-process host (the Nim cli, the C++ mirror): a group owns one context and one communicator rank per
  * device and runs every collective call on one worker thread per GPU.  Results are those of rank 0. */
