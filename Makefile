@@ -6,7 +6,7 @@ NVCCFLAGS := -gencode arch=compute_100a,code=sm_100a -O3 -lineinfo -std=c++17 -X
 all: lib cli oracle
 
 lib: $(PKG)/libcodexcommit.so
-$(PKG)/libcodexcommit.so: $(PKG)/csrc/capi.cu $(PKG)/csrc/kernels.cuh $(PKG)/csrc/poseidon2.cuh $(PKG)/csrc/fr.cuh $(PKG)/csrc/poseidon2_rc.cuh $(PKG)/csrc/fr_reduce_tab.cuh $(PKG)/csrc/capi_multi.cuh include/codex_commit.h
+$(PKG)/libcodexcommit.so: $(PKG)/csrc/capi.cu $(PKG)/csrc/kernels.cuh $(PKG)/csrc/poseidon2.cuh $(PKG)/csrc/fr.cuh $(PKG)/csrc/poseidon2_rc.cuh $(PKG)/csrc/fr_reduce_tab.cuh $(PKG)/csrc/capi_multi.cuh $(PKG)/csrc/slot_image.h include/codex_commit.h
 	$(NVCC) $(NVCCFLAGS) -o $@ $<
 
 cli: $(PKG)/cli

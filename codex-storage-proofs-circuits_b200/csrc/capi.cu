@@ -24,6 +24,7 @@
 #include <vector>
 
 #include "kernels.cuh"
+#include "slot_image.h"
 
 using namespace cdx;
 
@@ -603,11 +604,9 @@ extern "C" void cdx_slot_free(cdx_slot* s) {
 }
 
 static int check_shape(cdx_ctx* ctx, size_t n_bytes, size_t cell_size, size_t block_size) {
-  if (cell_size == 0 || cell_size % 4 || cell_size > (1u << 30)) return fail(ctx, CDX_ERR_SIZE, "cell size %zu must be a non-zero multiple of 4", cell_size);
-  if (block_size == 0 || block_size % cell_size) return fail(ctx, CDX_ERR_SIZE, "block size is not divisible by cell size");
-  if (!is_pow2(block_size / cell_size)) return fail(ctx, CDX_ERR_SIZE, "cells per block (%zu) must be a power of two", block_size / cell_size);
-  if (n_bytes == 0 || n_bytes % block_size) return fail(ctx, CDX_ERR_SIZE, "slot size %zu is not a non-zero multiple of the block size", n_bytes);
-  return CDX_OK;
+  char msg[128];
+  const int rc = slot_shape_status(n_bytes, cell_size, block_size, msg, sizeof msg);
+  return rc ? fail(ctx, rc, "%s", msg) : CDX_OK;
 }
 
 // allocate a slot handle and lay out its layers; on success the caller fills forest[0] and calls build_trees
@@ -1163,13 +1162,7 @@ extern "C" int cdx_slot_commit_fake(cdx_ctx* ctx, uint64_t seed, size_t n_cells,
 }
 
 // ---- persisted commitments ------------------------------------------------------------------------------------
-// A full image ("CDXSLOT1") holds the block forest and slot levels 1..depth; a compact image ("CDXSLOTC", forest_nodes = 0)
-// holds slot levels 0..depth, i.e. the block hashes and everything above them.
-struct SlotImageHeader {
-  char magic[8];              // "CDXSLOT1" or "CDXSLOTC"
-  uint64_t cell_size, block_size, n_blocks, forest_nodes, top_nodes;
-  uint32_t block_depth, slot_depth;
-};
+// The image format and the header checks of import are in slot_image.h.
 
 static size_t forest_node_count(const cdx_slot* s) {
   const uint64_t cpb = s->block_size / s->cell_size;
@@ -1222,31 +1215,52 @@ extern "C" int cdx_slot_export(const cdx_slot* s, uint8_t* image, size_t image_b
   return CDX_OK;
 }
 
+// The retained levels of an image that has just been copied to the device, checked in one launch of k_check_image: every
+// stored parent against its stored children, every element canonical.  CDX_ERR_MISMATCH names the smallest bad node.
+static int check_image_levels(cdx_slot* s) {
+  cdx_ctx* ctx = s->ctx;
+  ImageChain chain;
+  memset(&chain, 0, sizeof chain);
+  uint64_t total = 0;
+  auto add = [&](const uint8_t* nodes, uint64_t n, uint32_t tree, uint32_t level, uint32_t bottom, uint32_t singles) {
+    ImageLevel& L = chain.lv[chain.n_levels++];
+    L = ImageLevel{nodes, n, total, (uint8_t)tree, (uint8_t)level, (uint8_t)bottom, (uint8_t)singles};
+    total += n;
+  };
+  const bool singles = s->block_size / s->cell_size == 1;
+  if (!s->compact)
+    for (uint32_t l = 0; l <= s->block_depth; ++l) add(s->forest[l], singles ? s->n_local_cells : s->n_local_cells >> l, 0, l, l == 1, singles && l == 1);
+  else
+    add(s->top[0], s->width[0], 1, 0, 0, 0);
+  for (uint32_t l = 1; l <= s->slot_depth; ++l) add(s->top[l], s->width[l], 1, l, l == 1, 0);
+  DevBuf d_bad;
+  CU_TRY(ctx, d_bad.alloc(8, s->stream));
+  CU_TRY(ctx, cudaMemsetAsync(d_bad.p, 0xff, 8, s->stream));
+  LAUNCH(ctx, k_check_image, total, s->stream, chain, total, (unsigned long long*)d_bad.p);
+  unsigned long long bad = 0;
+  CU_TRY(ctx, cudaMemcpyAsync(&bad, d_bad.p, 8, cudaMemcpyDeviceToHost, s->stream));
+  CU_TRY(ctx, cudaStreamSynchronize(s->stream));
+  if (bad == ~0ull) return CDX_OK;
+  return fail(ctx, CDX_ERR_MISMATCH, "slot image: %s level %u node %llu %s", bad >> 63 ? "slot-tree" : "block-forest", (unsigned)(bad >> 57) & 63u,
+              (bad & ((1ull << 57) - 1)) >> 1, bad & 1 ? "does not hash from its children" : "is not canonical");
+}
+
 extern "C" int cdx_slot_import(cdx_ctx* ctx, const uint8_t* image, size_t image_bytes, cdx_slot** out) {
   if (!ctx || !image || !out) return fail(ctx, CDX_ERR_ARG, "null pointer");
   *out = nullptr;
-  SlotImageHeader h;
-  if (image_bytes < sizeof h) return fail(ctx, CDX_ERR_SIZE, "image too small");
-  memcpy(&h, image, sizeof h);
-  const bool compact = memcmp(h.magic, "CDXSLOTC", 8) == 0;
-  if (!compact && memcmp(h.magic, "CDXSLOT1", 8) != 0) return fail(ctx, CDX_ERR_ARG, "not a slot image");
-  int rc = check_shape(ctx, h.n_blocks * h.block_size, h.cell_size, h.block_size);
-  if (rc) return rc;
+  SlotImageLayout L;
+  char msg[200];
+  int rc = slot_image_layout(image, image_bytes, &L, msg, sizeof msg);
+  if (rc) return fail(ctx, rc, "%s", msg);
   CU_TRY(ctx, cudaSetDevice(ctx->device));
   cdx_slot* s = nullptr;
-  rc = slot_alloc(ctx, h.n_blocks, h.cell_size, h.block_size, 0, h.n_blocks, 0, ctx->stream, &s, false, compact);
+  rc = slot_alloc(ctx, L.n_blocks, L.cell_size, L.block_size, 0, L.n_blocks, 0, ctx->stream, &s, false, L.compact);
   if (rc) return rc;
   auto body = [&]() -> int {
-    if ((compact ? 0 : forest_node_count(s)) != h.forest_nodes || s->block_depth != h.block_depth || s->slot_depth != h.slot_depth)
-      return fail(ctx, CDX_ERR_ARG, "slot image header is inconsistent with its geometry");
-    size_t top_nodes = 0;
-    for (uint32_t l = 1; l <= s->slot_depth; ++l) top_nodes += s->width[l];
-    const size_t level0_nodes = compact ? s->width[0] : h.forest_nodes;   // what precedes slot level 1 in the payload
-    if (top_nodes != h.top_nodes || image_bytes != sizeof h + 32 * (level0_nodes + h.top_nodes)) return fail(ctx, CDX_ERR_SIZE, "slot image has the wrong length");
-    const uint8_t* p = image + sizeof h;
-    CU_TRY(ctx, cudaMemcpyAsync(s->d_forest, p, 32 * level0_nodes, cudaMemcpyHostToDevice, s->stream));
-    p += 32 * level0_nodes;
-    if (top_nodes) CU_TRY(ctx, dev_alloc((void**)&s->d_top, 32 * top_nodes, s->stream));
+    const uint8_t* p = image + sizeof(SlotImageHeader);
+    CU_TRY(ctx, cudaMemcpyAsync(s->d_forest, p, 32 * L.level0_nodes, cudaMemcpyHostToDevice, s->stream));
+    p += 32 * L.level0_nodes;
+    CU_TRY(ctx, dev_alloc((void**)&s->d_top, 32 * L.top_nodes, s->stream));
     s->top.assign(s->slot_depth + 1, nullptr);
     s->top[0] = s->low[0];
     size_t off = 0;
@@ -1254,11 +1268,10 @@ extern "C" int cdx_slot_import(cdx_ctx* ctx, const uint8_t* image, size_t image_
       s->top[l] = s->d_top + 32 * off;
       off += s->width[l];
     }
-    if (top_nodes) CU_TRY(ctx, cudaMemcpyAsync(s->d_top, p, 32 * top_nodes, cudaMemcpyHostToDevice, s->stream));
+    CU_TRY(ctx, cudaMemcpyAsync(s->d_top, p, 32 * L.top_nodes, cudaMemcpyHostToDevice, s->stream));
     s->top0_alias = true;
     s->has_top = true;
-    CU_TRY(ctx, cudaStreamSynchronize(s->stream));
-    return CDX_OK;
+    return check_image_levels(s);
   };
   rc = body();
   if (rc) {

@@ -206,16 +206,10 @@ __global__ void __launch_bounds__(CDX_BLOCK) k_compress_batch(const uint8_t* __r
   st_felt(out + 32 * i, from_mont(compress_keyed(to_mont(ld_felt(x + 32 * i)), to_mont(ld_felt(y + 32 * i)), keys[i] & 3u)));
 }
 
-// K3: one Merkle level.  out[i] = compress(in[2i], in[2i+1], bottom) ; a trailing single child is paired with 0
-// under key bottom+2 (merkle/bn254.nim:38-53, Merkle.hs:156-178).  The same kernel reduces the forest of block
-// trees (their widths are powers of two, so pairs never straddle two blocks) and every slot/dataset level.
-// singles != 0: every input is a one-leaf tree of its own -> out[i] = compress(in[i], 0, 3) (Merkle.hs:73).
-__global__ void __launch_bounds__(CDX_BLOCK) k_merkle_level(const uint8_t* __restrict__ in, size_t n, uint8_t* __restrict__ out,
-                                                            uint32_t bottom, int singles) {
-  CDX_KERNEL_PROLOGUE();
-  const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-  const size_t n_out = singles ? n : (n + 1) / 2;
-  if (i >= n_out) return;
+// The Merkle node rule: node i of the level above `in` (n nodes) = compress(in[2i], in[2i+1], bottom); a trailing single
+// child is paired with 0 under key bottom+2 (merkle/bn254.nim:38-53, Merkle.hs:156-178).  singles != 0: every input is a
+// one-leaf tree of its own -> node i = compress(in[i], 0, 3) (Merkle.hs:73).  Canonical standard form.
+static __device__ __forceinline__ Fr merkle_node(const uint8_t* __restrict__ in, size_t n, size_t i, uint32_t bottom, int singles) {
   Fr x, y;
   uint32_t key = bottom;
   if (singles) {
@@ -231,7 +225,78 @@ __global__ void __launch_bounds__(CDX_BLOCK) k_merkle_level(const uint8_t* __res
       key = bottom + 2u;
     }
   }
-  st_felt(out + 32 * i, from_mont(compress_keyed(x, y, key)));
+  return from_mont(compress_keyed(x, y, key));
+}
+
+// K3: one Merkle level, out[i] = merkle_node(in, n, i).  The same kernel reduces the forest of block trees (their widths
+// are powers of two, so pairs never straddle two blocks) and every slot/dataset level.
+__global__ void __launch_bounds__(CDX_BLOCK) k_merkle_level(const uint8_t* __restrict__ in, size_t n, uint8_t* __restrict__ out,
+                                                            uint32_t bottom, int singles) {
+  CDX_KERNEL_PROLOGUE();
+  const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  const size_t n_out = singles ? n : (n + 1) / 2;
+  if (i >= n_out) return;
+  st_felt(out + 32 * i, merkle_node(in, n, i, bottom, singles));
+}
+
+// ---- checking an imported slot image (cdx_slot_import) ------------------------------------------------------------------
+// The retained levels of an image form one chain, bottom up: a full image's block-forest levels 0..block_depth and then slot
+// levels 1..slot_depth (slot level 1 is built from the block hashes, forest level block_depth); a compact image's slot
+// levels 0..slot_depth.  Every stored node above the bottom level must be what the node rule makes of its stored children,
+// and every stored element must be canonical.  Both use stored values only, so one launch covers every level in place.
+#define CDX_IMAGE_LEVELS 72                    // 33 block-forest levels + slot levels 1..39 (slot_image.h)
+
+struct ImageLevel {
+  const uint8_t* nodes;
+  uint64_t n;                                  // nodes of this level
+  uint64_t first;                              // its first thread: the prefix sum of n over the levels below
+  uint8_t tree, level, bottom, singles;        // tree 0 = block forest, 1 = slot tree; node rule of the level below
+};
+
+struct ImageChain {
+  ImageLevel lv[CDX_IMAGE_LEVELS];
+  uint32_t n_levels;
+};
+
+static __device__ __forceinline__ bool fr_is_canonical(const Fr& a) {
+  const uint32_t r[8] = {CDX_N0, CDX_N1, CDX_N2, CDX_N3, CDX_N4, CDX_N5, CDX_N6, CDX_N7};
+#pragma unroll
+  for (int k = 7; k >= 0; --k)
+    if (a.l[k] != r[k]) return a.l[k] < r[k];
+  return false;
+}
+
+// the key of a bad node: smaller is (forest before slot tree, lower level, lower node, "not canonical" before "does not hash")
+static __host__ __device__ __forceinline__ unsigned long long image_bad_key(uint32_t tree, uint32_t level, uint64_t node, uint32_t hashes) {
+  return ((unsigned long long)tree << 63) | ((unsigned long long)level << 57) | (node << 1) | hashes;
+}
+
+// one thread per stored node (nodes < 2^56 a level: an image's levels are allocated in HBM); bad = the smallest key
+__global__ void __launch_bounds__(CDX_BLOCK) k_check_image(const __grid_constant__ ImageChain chain, uint64_t total, unsigned long long* __restrict__ bad) {
+  CDX_KERNEL_PROLOGUE();
+  const uint64_t t = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= total) return;
+  uint32_t lo = 0, hi = chain.n_levels;        // the level with first <= t < first + n
+  while (hi - lo > 1) {
+    const uint32_t mid = (lo + hi) >> 1;
+    if (chain.lv[mid].first <= t) lo = mid;
+    else hi = mid;
+  }
+  const ImageLevel& L = chain.lv[lo];
+  const uint64_t i = t - L.first;
+  const Fr v = ld_felt(L.nodes + 32 * i);
+  unsigned long long key = ~0ull;
+  if (!fr_is_canonical(v)) {
+    key = image_bad_key(L.tree, L.level, i, 0);
+  } else if (lo > 0) {
+    const ImageLevel& C = chain.lv[lo - 1];
+    const Fr h = merkle_node(C.nodes, C.n, i, L.bottom, L.singles);
+    bool same = true;
+#pragma unroll
+    for (int k = 0; k < 8; ++k) same &= h.l[k] == v.l[k];
+    if (!same) key = image_bad_key(L.tree, L.level, i, 1);
+  }
+  if (key != ~0ull) atomicMin(bad, key);
 }
 
 // elements in place to canonical standard form: any 256-bit input is taken mod r.  The bottom layer a caller hands to

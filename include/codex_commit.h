@@ -39,7 +39,8 @@ typedef enum cdx_status {
   CDX_ERR_CUDA = -5,     /* CUDA runtime error, or no device */
   CDX_ERR_ALLOC = -6,
   CDX_ERR_STATE = -7,    /* handle not in the state the call needs (e.g. sharded slot without its top tree) */
-  CDX_ERR_MISMATCH = -8  /* slot bytes do not hash to the retained commitment (cdx_slot_prove_from_source) */
+  CDX_ERR_MISMATCH = -8  /* slot bytes do not hash to the retained commitment (cdx_slot_prove_from_source), or a node
+                            of a slot image does not hash from its children or is not canonical (cdx_slot_import) */
 } cdx_status;
 
 typedef struct cdx_ctx cdx_ctx;   /* per-GPU context: device, streams, staging buffers */
@@ -151,12 +152,21 @@ int cdx_slot_set_top_dev(cdx_slot* slot, const void* d_level_nodes, uint64_t n_l
 
 /* Persist / restore a commitment (SURVEY.md 8f item 2: a proof server answers repeated challenges from a retained
  * commitment instead of re-hashing the slot).  The image is a small header followed by every retained layer (canonical
- * 32-byte elements), about 3.1 % of the slot size; it is self-describing and checked on import.  Only whole
+ * 32-byte elements), about 3.1 % of the slot size; it is self-describing.  Only whole
  * (non-sharded, top tree present) slots can be exported.  The reference keeps nothing: it rebuilds the slot tree for
  * every sample (nim/gen_input/bn254.nim:57).
  * A compact slot (cdx_slot_compact) exports a compact image: magic "CDXSLOTC", forest_nodes = 0, slot-tree levels
  * 0..slot_tree_depth (32 bytes x the sum of their widths, about 0.1 % of the slot at the default geometry); importing it
- * gives a compact slot. */
+ * gives a compact slot.
+ * Import checks the image before it returns a handle.  First the header, before anything is allocated: the magic
+ * (CDX_ERR_ARG); the cell and block sizes as a commit checks them and sizes that would overflow 64 bits (CDX_ERR_SIZE);
+ * depths and forest_nodes that disagree with the geometry (CDX_ERR_ARG); trees deeper than a proof call can answer for,
+ * block_tree_depth > 32 or slot_tree_depth > 39 (CDX_ERR_RANGE); top_nodes and the image length (CDX_ERR_SIZE).
+ * Then the payload, on the device:
+ * every stored node above the bottom level must be the compression of its stored children, and every stored element
+ * must be canonical (< r); otherwise CDX_ERR_MISMATCH, and the message names the smallest bad node (tree, level, node).
+ * So an imported slot is internally consistent; that its root is the root the caller expects is for the caller to
+ * compare (cdx_slot_root). */
 size_t cdx_slot_export_size(const cdx_slot* slot);
 int cdx_slot_export(const cdx_slot* slot, uint8_t* image, size_t image_bytes);
 int cdx_slot_import(cdx_ctx* ctx, const uint8_t* image, size_t image_bytes, cdx_slot** out);
