@@ -15,6 +15,6 @@ The directory name is not a Python identifier; import it with
 (tests/conftest.py and bench.py do exactly that).
 """
 from . import capi  # noqa: F401
-from .capi import CodexCommitError, Comm, Context, Dataset, Slot, load_library  # noqa: F401
+from .capi import CodexCommitError, Comm, Context, Dataset, Slot, SlotBuilder, load_library  # noqa: F401
 
-__all__ = ["capi", "Context", "Slot", "Comm", "Dataset", "CodexCommitError", "load_library"]
+__all__ = ["capi", "Context", "Slot", "SlotBuilder", "Comm", "Dataset", "CodexCommitError", "load_library"]

@@ -9,7 +9,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libcodexcommit.so")
 SOURCES = ["capi.cu"]
-HEADERS = ["fr.cuh", "fr_reduce_tab.cuh", "poseidon2.cuh", "poseidon2_rc.cuh", "kernels.cuh", "capi_multi.cuh", "slot_image.h", os.path.join("..", "..", "include", "codex_commit.h")]
+HEADERS = ["fr.cuh", "fr_reduce_tab.cuh", "poseidon2.cuh", "poseidon2_rc.cuh", "kernels.cuh", "capi_multi.cuh", "slot_image.h", "slot_builder.h",os.path.join("..", "..", "include", "codex_commit.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "-Xcompiler", "-fPIC",
               "-shared", "-ldl"]
 

@@ -95,6 +95,10 @@ SYMBOLS = {
     "cdx_slot_device_bytes": (_sz, [_vp]),
     "cdx_slot_prove_from_source": (_int, [_vp, _vp, _vp, _sz, _sz, _sz, _vp, _vp, _vp, _vp]),
     "cdx_slots_prove_from_source": (_int, [_vp, _vp, _vp, _sz, _sz, _sz, _vp, _vp, _vp, _vp]),
+    "cdx_slot_builder_create": (_int, [_vp, _u64, _sz, _sz, _int, _pp]),
+    "cdx_slot_builder_add_host": (_int, [_vp, _u64, _vp, _sz]),
+    "cdx_slot_builder_finish": (_int, [_vp, _pp]),
+    "cdx_slot_builder_free": (None, [_vp]),
     "cdx_group_create": (_int, [C.POINTER(_int), _int, _pp]),
     "cdx_group_destroy": (None, [_vp]),
     "cdx_group_size": (_int, [_vp]),
@@ -436,6 +440,13 @@ class Context:
         self._chk(self.lib.cdx_slot_commit_file(self.h, os.fsencode(path), offset, n_bytes, cell_size, block_size, C.byref(h)))
         return Slot(self, h)
 
+    def slot_builder(self, n_blocks: int, cell_size: int = 2048, block_size: int = 65536, keep_forest: bool = False) -> "SlotBuilder":
+        """a slot of n_blocks blocks committed from blocks added in any order (cdx_slot_builder_create); finish() returns a
+        full handle with keep_forest, else a compact one"""
+        h = C.c_void_p()
+        self._chk(self.lib.cdx_slot_builder_create(self.h, n_blocks, cell_size, block_size, int(bool(keep_forest)), C.byref(h)))
+        return SlotBuilder(self, h, block_size)
+
     def slot_import(self, image: bytes) -> "Slot":
         h = C.c_void_p()
         self._chk(self.lib.cdx_slot_import(self.h, _addr(image), len(image), C.byref(h)))
@@ -653,6 +664,43 @@ class Slot:
         return ([ii[j * n_samples:(j + 1) * n_samples] for j in range(k)],
                 [paths[j * n_samples:(j + 1) * n_samples] for j in range(k)],
                 [leaves[j * n_samples:(j + 1) * n_samples] for j in range(k)])
+
+
+class SlotBuilder:
+    """A slot being committed from blocks added in any order and in any number of pieces (cdx_slot_builder)."""
+
+    def __init__(self, ctx: Context, h, block_size: int):
+        self.ctx, self.h, self.block_size = ctx, h, block_size
+
+    def add(self, first_block: int, data, n_bytes: Optional[int] = None):
+        """blocks [first_block, first_block + n_bytes / block_size) from `data` (what _addr takes); the buffer may be reused
+        as soon as the call returns"""
+        nb = n_bytes if n_bytes is not None else (data.nbytes if hasattr(data, "nbytes") else len(data))
+        keep = data                      # keep the buffer alive for the duration of the call
+        self.ctx._chk(self.ctx.lib.cdx_slot_builder_add_host(self.h, first_block, _addr(keep), nb))
+
+    def finish(self) -> Slot:
+        """the committed slot; raises (and stays usable) while blocks are missing"""
+        h = C.c_void_p()
+        self.ctx._chk(self.ctx.lib.cdx_slot_builder_finish(self.h, C.byref(h)))
+        return Slot(self.ctx, h)
+
+    def free(self):
+        if getattr(self, "h", None):
+            self.ctx.lib.cdx_slot_builder_free(self.h)
+            self.h = None
+
+    def __del__(self):
+        try:
+            self.free()
+        except Exception:
+            pass
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *a):
+        self.free()
 
 
 class Comm:

@@ -24,6 +24,7 @@
 #include <vector>
 
 #include "kernels.cuh"
+#include "slot_builder.h"
 #include "slot_image.h"
 
 using namespace cdx;
@@ -690,19 +691,27 @@ static int slot_alloc(cdx_ctx* ctx, uint64_t n_local_blocks, size_t cell_size, s
   return CDX_OK;
 }
 
+// The block trees over n_cells cell hashes of whole blocks in forest[0]: levels 1..block_depth into forest[1..block_depth],
+// one launch per level (one launch for one-cell blocks, whose single level is one key-3 compression per cell).
+static int launch_block_trees(cdx_ctx* ctx, uint8_t* const* forest, size_t n_cells, bool singles, uint32_t block_depth, cudaStream_t st) {
+  if (singles) {
+    LAUNCH(ctx, k_merkle_level, n_cells, st, forest[0], n_cells, forest[1], 1u, 1);
+  } else {
+    for (uint32_t l = 0; l < block_depth; ++l) {
+      const size_t n = n_cells >> l;
+      LAUNCH(ctx, k_merkle_level, n / 2, st, forest[l], n, forest[l + 1], l == 0 ? 1u : 0u, 0);
+    }
+  }
+  return CDX_OK;
+}
+
 // block forest + local slot levels, assuming forest[0] (cell hashes) is already being produced on s->stream
 static int build_local_trees(cdx_slot* s) {
   cdx_ctx* ctx = s->ctx;
   const bool singles = (s->block_size / s->cell_size) == 1;
   if (s->n_local_cells == 0) return CDX_OK;                                  // empty shard
-  if (singles) {
-    LAUNCH(ctx, k_merkle_level, s->n_local_cells, s->stream, s->forest[0], (size_t)s->n_local_cells, s->forest[1], 1u, 1);
-  } else {
-    for (uint32_t l = 0; l < s->block_depth; ++l) {
-      const size_t n = s->n_local_cells >> l;
-      LAUNCH(ctx, k_merkle_level, n / 2, s->stream, s->forest[l], n, s->forest[l + 1], l == 0 ? 1u : 0u, 0);
-    }
-  }
+  int rc = launch_block_trees(ctx, s->forest.data(), (size_t)s->n_local_cells, singles, s->block_depth, s->stream);
+  if (rc) return rc;
   for (uint32_t l = 0; l < s->top_level; ++l) {
     const size_t n = s->low_count[l];
     LAUNCH(ctx, k_merkle_level, (n + 1) / 2, s->stream, s->low[l], n, s->low[l + 1], l == 0 ? 1u : 0u, 0);
@@ -955,6 +964,20 @@ static int hash_cells_pinned(cdx_ctx* ctx, const uint8_t* data, size_t n_bytes, 
                    d_hashes);
 }
 
+// len bytes of a source at offset off into dst through `fill`, split evenly over host threads (8 on a host with 16 or more
+// hardware threads, 4 with 8 or more, else 2): one thread copying pageable memory into pinned memory does not keep up
+// with the cell sponge.
+static void fill_chunk_parallel(const ChunkFill& fill, uint8_t* dst, uint64_t off, size_t len) {
+  const unsigned hw = std::thread::hardware_concurrency();
+  const unsigned n_thr = hw >= 16 ? 8 : (hw >= 8 ? 4 : 2);
+  std::vector<std::thread> thr;
+  for (unsigned t = 0; t < n_thr; ++t) {
+    const size_t a = len * t / n_thr, b = len * (t + 1) / n_thr;
+    if (b > a) thr.emplace_back([&fill, dst, off, a, b]() { fill(dst + a, off + a, b - a); });
+  }
+  for (auto& t : thr) t.join();
+}
+
 // Slot bytes that are not directly DMA-able (a file, or pageable host memory -- what a Nim seq[byte] is).  Host threads
 // fill one of two pinned chunks through `fill(dst, offset, len)` while the copy stream moves the other one into the
 // device tile; a tile is four chunks, copied on the one copy stream into two device buffers.
@@ -980,16 +1003,6 @@ static int hash_cells_staged(cdx_ctx* ctx, size_t n_bytes, size_t cell_size, siz
   }
   int rc = ensure_stage(ctx, tile_bytes);
   if (rc) return rc;
-  unsigned hw = std::thread::hardware_concurrency();
-  const unsigned n_thr = hw >= 16 ? 8 : (hw >= 8 ? 4 : 2);
-  auto fill_chunk_parallel = [&](uint8_t* dst, uint64_t off, size_t len) {
-    std::vector<std::thread> thr;
-    for (unsigned t = 0; t < n_thr; ++t) {
-      const size_t a = len * t / n_thr, b = len * (t + 1) / n_thr;
-      if (b > a) thr.emplace_back([&fill, dst, off, a, b]() { fill(dst + a, off + a, b - a); });
-    }
-    for (auto& t : thr) t.join();
-  };
   // tile 0 is one chunk, tile 1 the other three: the sponge starts after one chunk has been filled and copied, not four
   std::vector<size_t> head;
   if (n_blocks > tile_blocks && tile_blocks > chunk_blocks) head = {chunk_blocks, tile_blocks - chunk_blocks};
@@ -999,7 +1012,7 @@ static int hash_cells_staged(cdx_ctx* ctx, size_t n_bytes, size_t cell_size, siz
       const int pb = (int)(chunk_no & 1);
       const size_t cnb = nb - cb < chunk_blocks ? nb - cb : chunk_blocks;
       if (chunk_no >= 2) CU_TRY(ctx, cudaEventSynchronize(ctx->ev_h2d[pb]));                  // pinned chunk pb drained
-      fill_chunk_parallel((uint8_t*)ctx->h_pinned[pb], (uint64_t)(first + cb) * block_size, cnb * block_size);
+      fill_chunk_parallel(fill, (uint8_t*)ctx->h_pinned[pb], (uint64_t)(first + cb) * block_size, cnb * block_size);
       CU_TRY(ctx, cudaMemcpyAsync(dst + cb * block_size, ctx->h_pinned[pb], cnb * block_size, cudaMemcpyHostToDevice, cp));
       CU_TRY(ctx, cudaEventRecord(ctx->ev_h2d[pb], cp));
     }
@@ -1159,6 +1172,290 @@ extern "C" int cdx_slot_commit_fake(cdx_ctx* ctx, uint64_t seed, size_t n_cells,
   src.kind = CDX_SRC_FAKE;
   src.seed = seed;
   return commit_from_source(ctx, src, n_cells * cell_size, cell_size, block_size, 0, 0, 0, true, true, out);
+}
+
+// ---- slot builder: a slot's blocks added in any order and in any number of pieces --------------------------------------
+// The caller's bytes are copied into a ring of four pinned chunks (a quarter tile each); a chunk is copied to the device
+// tile as soon as it is full, while the next one fills.  A full tile (tile_blocks blocks, the tile of hash_cells_staged) is
+// hashed by the cell sponge, its block trees are built in a scratch forest and the results are scattered to their blocks'
+// places in the handle: every forest level of a full handle, the block hashes of a compact one.  Two device tiles, each
+// with its own compute stream, so that the kernels of one tile overlap the filling of the next.  Adds that do not complete
+// a tile launch nothing.  The builder owns its streams and buffers: ctx->d_stage and ctx->h_pinned are shared with every
+// other call on the context, so other calls may run between two adds.  The bookkeeping is in slot_builder.h.
+#define CDX_BUILDER_CHUNKS 4
+
+struct cdx_slot_builder {
+  cdx_ctx* ctx = nullptr;
+  cdx_slot* slot = nullptr;              // the handle being filled; a compact one has no forest below the block hashes
+  SlotBuilderBook book;
+  size_t cell_size = 0, block_size = 0, cpb = 0;
+  size_t tile_blocks = 0, chunk_blocks = 0;
+  uint64_t tiles = 0;                    // tiles flushed so far: the tile being filled goes to device tile tiles & 1
+  size_t pos = 0;                        // blocks of the current tile in the pinned chunks
+  size_t queued = 0;                     // ... of which the copy to the device tile has been queued
+  int error = CDX_OK;                    // an earlier call failed on the device: the builder refuses everything after it
+  std::vector<uint64_t> ids;             // the block at each position of the current tile
+  cudaStream_t copy = nullptr, compute[2] = {nullptr, nullptr};
+  cudaEvent_t ev_chunk[CDX_BUILDER_CHUNKS] = {};   // the last copy out of pinned chunk c
+  cudaEvent_t ev_copied[2] = {}, ev_consumed[2] = {}, ev_join = nullptr;
+  uint8_t* h_chunk[CDX_BUILDER_CHUNKS] = {};
+  uint64_t* h_ids[2] = {nullptr, nullptr};         // pinned: the block-id table of device tile t on its way up
+  DevBuf d_tile[2], d_ids[2], d_forest[2];
+  std::vector<uint8_t*> forest[2];                 // the scratch forest's levels 0..block_depth, per device tile
+};
+
+static constexpr size_t kBuilderParallelFill = (size_t)4 << 20;   // pieces from this size on are copied by several host threads
+
+// The builder's own streams, events and buffers, released in every state (the slot being built is not among them).
+static void builder_release(cdx_slot_builder* b) {
+  cudaSetDevice(b->ctx->device);
+  for (cudaStream_t s : {b->copy, b->compute[0], b->compute[1]})
+    if (s) cudaStreamSynchronize(s);
+  for (int t = 0; t < 2; ++t)
+    for (DevBuf* d : {&b->d_tile[t], &b->d_ids[t], &b->d_forest[t]}) {
+      if (d->p) dev_free(d->p, d->st);
+      d->p = nullptr;
+    }
+  for (int c = 0; c < CDX_BUILDER_CHUNKS; ++c) {
+    if (b->h_chunk[c]) cudaFreeHost(b->h_chunk[c]);
+    if (b->ev_chunk[c]) cudaEventDestroy(b->ev_chunk[c]);
+    b->h_chunk[c] = nullptr;
+    b->ev_chunk[c] = nullptr;
+  }
+  for (int t = 0; t < 2; ++t) {
+    if (b->h_ids[t]) cudaFreeHost(b->h_ids[t]);
+    if (b->ev_copied[t]) cudaEventDestroy(b->ev_copied[t]);
+    if (b->ev_consumed[t]) cudaEventDestroy(b->ev_consumed[t]);
+    b->h_ids[t] = nullptr;
+    b->ev_copied[t] = b->ev_consumed[t] = nullptr;
+    b->forest[t].clear();
+  }
+  if (b->ev_join) cudaEventDestroy(b->ev_join);
+  b->ev_join = nullptr;
+  for (cudaStream_t* s : {&b->copy, &b->compute[0], &b->compute[1]}) {
+    if (*s) cudaStreamDestroy(*s);
+    *s = nullptr;
+  }
+  std::vector<uint64_t>().swap(b->ids);
+}
+
+static int builder_setup(cdx_slot_builder* b, uint64_t n_blocks, bool compact) {
+  cdx_ctx* ctx = b->ctx;
+  size_t tile_blocks = (ctx->tile_mib << 20) / b->block_size;
+  if (tile_blocks == 0) tile_blocks = 1;
+  if (tile_blocks > n_blocks) tile_blocks = n_blocks;
+  b->tile_blocks = tile_blocks;
+  b->chunk_blocks = (tile_blocks + CDX_BUILDER_CHUNKS - 1) / CDX_BUILDER_CHUNKS;
+  int rc = slot_alloc(ctx, n_blocks, b->cell_size, b->block_size, 0, n_blocks, 0, ctx->stream, &b->slot, false, compact);
+  if (rc) return rc;
+  try {
+    slot_builder_init(&b->book, n_blocks);
+    b->ids.assign(tile_blocks, 0);
+  } catch (const std::bad_alloc&) {
+    return fail(ctx, CDX_ERR_ALLOC, "host allocation of the bookkeeping of %llu blocks failed", (unsigned long long)n_blocks);
+  }
+  for (cudaStream_t* s : {&b->copy, &b->compute[0], &b->compute[1]}) CU_TRY(ctx, cudaStreamCreateWithFlags(s, cudaStreamNonBlocking));
+  for (int c = 0; c < CDX_BUILDER_CHUNKS; ++c) CU_TRY(ctx, cudaEventCreateWithFlags(&b->ev_chunk[c], cudaEventDisableTiming));
+  for (int t = 0; t < 2; ++t) {
+    CU_TRY(ctx, cudaEventCreateWithFlags(&b->ev_copied[t], cudaEventDisableTiming));
+    CU_TRY(ctx, cudaEventCreateWithFlags(&b->ev_consumed[t], cudaEventDisableTiming));
+  }
+  CU_TRY(ctx, cudaEventCreateWithFlags(&b->ev_join, cudaEventDisableTiming));
+  // the handle's levels were allocated on ctx->stream, the builder's buffers are allocated on compute[0]
+  CU_TRY(ctx, cudaEventRecord(b->ev_join, ctx->stream));
+  CU_TRY(ctx, cudaStreamWaitEvent(b->compute[0], b->ev_join, 0));
+  const size_t tile_cells = tile_blocks * b->cpb;
+  const uint32_t bd = b->slot->block_depth;
+  std::vector<size_t> f_off;
+  size_t forest_nodes = 0;
+  for (uint32_t l = 0; l <= bd; ++l) {
+    f_off.push_back(forest_nodes);
+    forest_nodes += b->cpb == 1 ? tile_cells : (tile_cells >> l);
+  }
+  for (int t = 0; t < 2; ++t) {
+    if (b->d_tile[t].alloc(tile_blocks * b->block_size, b->compute[0]) != cudaSuccess || b->d_ids[t].alloc(8 * tile_blocks, b->compute[0]) != cudaSuccess ||
+        b->d_forest[t].alloc(32 * forest_nodes, b->compute[0]) != cudaSuccess)
+      return fail(ctx, CDX_ERR_ALLOC, "cudaMalloc of the slot builder's tiles failed");
+    for (uint32_t l = 0; l <= bd; ++l) b->forest[t].push_back(b->d_forest[t].u8() + 32 * f_off[l]);
+  }
+  CU_TRY(ctx, cudaEventRecord(b->ev_join, b->compute[0]));
+  CU_TRY(ctx, cudaStreamWaitEvent(b->copy, b->ev_join, 0));
+  CU_TRY(ctx, cudaStreamWaitEvent(b->compute[1], b->ev_join, 0));
+  const size_t n_chunks = (tile_blocks + b->chunk_blocks - 1) / b->chunk_blocks;
+  for (size_t c = 0; c < n_chunks; ++c)
+    if (cudaHostAlloc((void**)&b->h_chunk[c], b->chunk_blocks * b->block_size, cudaHostAllocDefault) != cudaSuccess)
+      return fail(ctx, CDX_ERR_ALLOC, "cudaHostAlloc of %zu bytes failed", b->chunk_blocks * b->block_size);
+  for (int t = 0; t < 2; ++t)
+    if (cudaHostAlloc((void**)&b->h_ids[t], 8 * tile_blocks, cudaHostAllocDefault) != cudaSuccess)
+      return fail(ctx, CDX_ERR_ALLOC, "cudaHostAlloc of %zu bytes failed", 8 * tile_blocks);
+  return CDX_OK;
+}
+
+extern "C" int cdx_slot_builder_create(cdx_ctx* ctx, uint64_t n_blocks, size_t cell_size, size_t block_size, int keep_forest, cdx_slot_builder** out) {
+  if (!ctx || !out) return fail(ctx, CDX_ERR_ARG, "null pointer");
+  *out = nullptr;
+  char msg[160];
+  int rc = slot_builder_shape(n_blocks, cell_size, block_size, msg, sizeof msg);
+  if (rc) return fail(ctx, rc, "%s", msg);
+  CU_TRY(ctx, cudaSetDevice(ctx->device));
+  cdx_slot_builder* b = new (std::nothrow) cdx_slot_builder();
+  if (!b) return fail(ctx, CDX_ERR_ALLOC, "host allocation failed");
+  b->ctx = ctx;
+  b->cell_size = cell_size;
+  b->block_size = block_size;
+  b->cpb = block_size / cell_size;
+  rc = builder_setup(b, n_blocks, keep_forest == 0);
+  if (rc) {
+    cdx_slot_builder_free(b);
+    return rc;
+  }
+  *out = b;
+  return CDX_OK;
+}
+
+// queue the copy of the pinned chunk being filled (blocks [queued, pos) of the current tile) to the device tile
+static int builder_copy_chunk(cdx_slot_builder* b) {
+  cdx_ctx* ctx = b->ctx;
+  if (b->pos == b->queued) return CDX_OK;
+  const int t = (int)(b->tiles & 1);
+  if (b->queued == 0) CU_TRY(ctx, cudaStreamWaitEvent(b->copy, b->ev_consumed[t], 0));   // the tile before last is out of device tile t
+  const size_t c = b->queued / b->chunk_blocks;
+  CU_TRY(ctx, cudaMemcpyAsync(b->d_tile[t].u8() + b->queued * b->block_size, b->h_chunk[c], (b->pos - b->queued) * b->block_size,
+                              cudaMemcpyHostToDevice, b->copy));
+  CU_TRY(ctx, cudaEventRecord(b->ev_chunk[c], b->copy));
+  b->queued = b->pos;
+  return CDX_OK;
+}
+
+static int launch_scatter_felts(cdx_ctx* ctx, const uint8_t* src, const uint64_t* index, size_t n, uint8_t* dst, uint32_t width, cudaStream_t st) {
+  k_scatter_felts<<<grid_for(2 * n * width, 256), 256, 0, st>>>(src, index, n, dst, width);
+  ctx->launches++;
+  CU_TRY(ctx, cudaGetLastError());
+  return CDX_OK;
+}
+
+// The current tile (pos blocks) through the cell sponge, its block trees and the scatter into the handle, on the compute
+// stream of its device tile.
+static int builder_flush(cdx_slot_builder* b) {
+  cdx_ctx* ctx = b->ctx;
+  cdx_slot* s = b->slot;
+  int rc = builder_copy_chunk(b);
+  if (rc) return rc;
+  const int t = (int)(b->tiles & 1);
+  const size_t nb = b->pos, n_cells = nb * b->cpb;
+  const uint32_t bd = s->block_depth;
+  CU_TRY(ctx, cudaEventSynchronize(b->ev_copied[t]));                 // the previous table uploaded from h_ids[t] has left it
+  memcpy(b->h_ids[t], b->ids.data(), 8 * nb);
+  CU_TRY(ctx, cudaMemcpyAsync(b->d_ids[t].p, b->h_ids[t], 8 * nb, cudaMemcpyHostToDevice, b->copy));
+  CU_TRY(ctx, cudaEventRecord(b->ev_copied[t], b->copy));
+  cudaStream_t cs = b->compute[t];
+  CU_TRY(ctx, cudaStreamWaitEvent(cs, b->ev_copied[t], 0));
+  rc = launch_hash_cells(ctx, b->d_tile[t].p, n_cells, b->cell_size, b->forest[t][0], cs);
+  if (rc) return rc;
+  rc = launch_block_trees(ctx, b->forest[t].data(), n_cells, b->cpb == 1, bd, cs);
+  if (rc) return rc;
+  const uint64_t* ids = (const uint64_t*)b->d_ids[t].p;
+  if (s->compact) {
+    rc = launch_scatter_felts(ctx, b->forest[t][bd], ids, nb, s->forest[bd], 1, cs);
+    if (rc) return rc;
+  } else {
+    for (uint32_t l = 0; l <= bd; ++l) {                                // level l of block k: cpb >> l nodes from k * (cpb >> l)
+      rc = launch_scatter_felts(ctx, b->forest[t][l], ids, nb, s->forest[l], b->cpb == 1 ? 1u : (uint32_t)(b->cpb >> l), cs);
+      if (rc) return rc;
+    }
+  }
+  CU_TRY(ctx, cudaEventRecord(b->ev_consumed[t], cs));
+  ++b->tiles;
+  b->pos = b->queued = 0;
+  return CDX_OK;
+}
+
+// blocks [first, first + n) from data, already checked and marked
+static int builder_take(cdx_slot_builder* b, uint64_t first, const uint8_t* data, uint64_t n) {
+  cdx_ctx* ctx = b->ctx;
+  const size_t bs = b->block_size;
+  while (n) {
+    const size_t c = b->pos / b->chunk_blocks, in = b->pos % b->chunk_blocks;
+    const size_t chunk_end = std::min((c + 1) * b->chunk_blocks, b->tile_blocks);
+    const size_t m = (size_t)std::min<uint64_t>(n, chunk_end - b->pos);
+    if (in == 0) CU_TRY(ctx, cudaEventSynchronize(b->ev_chunk[c]));     // the chunk's last copy has left it (never recorded = done)
+    uint8_t* dst = b->h_chunk[c] + in * bs;
+    if (m * bs >= kBuilderParallelFill) {
+      const ChunkFill fill = [data](uint8_t* d, uint64_t off, size_t len) { memcpy(d, data + off, len); };
+      fill_chunk_parallel(fill, dst, 0, m * bs);
+    } else {
+      memcpy(dst, data, m * bs);
+    }
+    for (size_t k = 0; k < m; ++k) b->ids[b->pos + k] = first + k;
+    b->pos += m;
+    first += m;
+    data += m * bs;
+    n -= m;
+    int rc = b->pos == chunk_end ? builder_copy_chunk(b) : CDX_OK;
+    if (rc == CDX_OK && b->pos == b->tile_blocks) rc = builder_flush(b);
+    if (rc) return rc;
+  }
+  return CDX_OK;
+}
+
+extern "C" int cdx_slot_builder_add_host(cdx_slot_builder* b, uint64_t first_block, const uint8_t* data, size_t n_bytes) {
+  if (!b) return CDX_ERR_ARG;
+  cdx_ctx* ctx = b->ctx;
+  if (!data) return fail(ctx, CDX_ERR_ARG, "null pointer");
+  if (b->error) return fail(ctx, CDX_ERR_STATE, "slot builder: an earlier call failed on the device, the builder cannot continue");
+  CU_TRY(ctx, cudaSetDevice(ctx->device));
+  char msg[160];
+  uint64_t n = 0;
+  int rc = slot_builder_add(&b->book, first_block, n_bytes, b->block_size, &n, msg, sizeof msg);
+  if (rc) return fail(ctx, rc, "%s", msg);
+  rc = builder_take(b, first_block, data, n);
+  if (rc) b->error = rc;
+  return rc;
+}
+
+extern "C" int cdx_slot_builder_finish(cdx_slot_builder* b, cdx_slot** out) {
+  if (!b) return CDX_ERR_ARG;
+  cdx_ctx* ctx = b->ctx;
+  if (!out) return fail(ctx, CDX_ERR_ARG, "null pointer");
+  *out = nullptr;
+  if (b->error) return fail(ctx, CDX_ERR_STATE, "slot builder: an earlier call failed on the device, the builder cannot continue");
+  char msg[160];
+  int rc = slot_builder_finish_status(&b->book, msg, sizeof msg);
+  if (rc) return fail(ctx, rc, "%s", msg);
+  cdx_slot* s = b->slot;
+  auto body = [&]() -> int {
+    CU_TRY(ctx, cudaSetDevice(ctx->device));
+    if (b->pos) {
+      int r = builder_flush(b);
+      if (r) return r;
+    }
+    for (int t = 0; t < 2; ++t) {                                       // the slot tree on the handle's stream, after both tiles
+      CU_TRY(ctx, cudaEventRecord(b->ev_join, b->compute[t]));
+      CU_TRY(ctx, cudaStreamWaitEvent(s->stream, b->ev_join, 0));
+    }
+    int r = build_top(s, s->low[0], true);
+    if (r) return r;
+    CU_TRY(ctx, cudaStreamSynchronize(s->stream));
+    return CDX_OK;
+  };
+  rc = body();
+  if (rc) {
+    b->error = rc;
+    return rc;
+  }
+  b->slot = nullptr;
+  b->book.finished = true;
+  std::vector<uint64_t>().swap(b->book.bits);
+  builder_release(b);
+  *out = s;
+  return CDX_OK;
+}
+
+extern "C" void cdx_slot_builder_free(cdx_slot_builder* b) {
+  if (!b) return;
+  builder_release(b);
+  if (b->slot) cdx_slot_free(b->slot);
+  delete b;
 }
 
 // ---- persisted commitments ------------------------------------------------------------------------------------
@@ -1835,14 +2132,8 @@ static int prove_rows(const cdx_slot* const* slots, const cdx_slot_desc* sources
                               cells_out ? &gather : nullptr);
       if (rc) return rc;
     }
-    if (cpb == 1) {
-      LAUNCH(ctx, k_merkle_level, n_cells, st, forest[0], n_cells, forest[1], 1u, 1);
-    } else {
-      for (uint32_t l = 0; l < block_depth; ++l) {
-        const size_t n = n_cells >> l;
-        LAUNCH(ctx, k_merkle_level, n / 2, st, forest[l], n, forest[l + 1], l == 0 ? 1u : 0u, 0);
-      }
-    }
+    rc = launch_block_trees(ctx, forest.data(), n_cells, cpb == 1, block_depth, st);
+    if (rc) return rc;
     // 6. every recomputed block hash against its slot's retained one
     CU_TRY(ctx, d_bad.alloc(8, st));
     CU_TRY(ctx, cudaMemsetAsync(d_bad.p, 0xff, 8, st));

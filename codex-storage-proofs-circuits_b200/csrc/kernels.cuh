@@ -339,12 +339,15 @@ __global__ void __launch_bounds__(CDX_BLOCK) k_merkle_level_seg(const uint8_t* _
   if (out_off[lo + 1] - out_off[lo] == 1) st_felt(roots + 32 * (size_t)lo, h);
 }
 
-// dst[index[i]] = src[i] for 32-byte elements (the roots of a batch of slots into their places among a dataset's slot roots)
-__global__ void k_scatter_felts(const uint8_t* __restrict__ src, const uint64_t* __restrict__ index, size_t n, uint8_t* __restrict__ dst) {
+// Runs of `width` 32-byte elements: run i of src goes to run index[i] of dst, dst[index[i] * width + k] = src[i * width + k].
+// Width 1 moves the roots of a batch of slots into their places among a dataset's slot roots; a slot builder moves each
+// level of a tile's block trees (width = that level's nodes per block) into the slot's forest.  One thread per 16-byte half.
+__global__ void k_scatter_felts(const uint8_t* __restrict__ src, const uint64_t* __restrict__ index, size_t n, uint8_t* __restrict__ dst,
+                                uint32_t width = 1) {
   const size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (t >= 2 * n) return;
-  const size_t i = t >> 1, half = t & 1;
-  reinterpret_cast<uint4*>(dst + 32 * index[i])[half] = reinterpret_cast<const uint4*>(src + 32 * i)[half];
+  if (t >= 2 * n * width) return;
+  const size_t e = t >> 1, half = t & 1, i = e / width, k = e - i * width;
+  reinterpret_cast<uint4*>(dst + 32 * (index[i] * width + k))[half] = reinterpret_cast<const uint4*>(src + 32 * e)[half];
 }
 
 // K4: batched path gather.  One thread per (sample, level, 16-byte half).  Pure data movement.

@@ -373,6 +373,52 @@ int cdx_slots_prove_from_source(const cdx_slot* const* slots, const cdx_slot_des
                                 size_t n_challenges, size_t n_samples, size_t max_depth, uint64_t* indices_out,
                                 uint8_t* paths_out, uint8_t* leaves_out, uint8_t* cells_out);
 
+/* ---- slot builder: a slot committed from blocks added in any order ------------------------------------------
+ * A storage node receives a slot's blocks one at a time or in short runs, from several peers, in whatever order they
+ * arrive.  A builder takes them as they come and hashes them while more arrive, so the slot is never staged whole in host
+ * memory and the hashing overlaps the download.  Replaces nothing in the reference, which loads whole slots
+ * (nim/slot.nim:51-73).
+ *
+ * cdx_slot_builder_create: the slot's shape up front, n_blocks blocks of block_size bytes; the shape rules are those of
+ * cdx_slot_commit_host on n_blocks * block_size bytes (CDX_ERR_SIZE, also when that product overflows 64 bits).
+ * keep_forest != 0: finish returns a full handle; keep_forest == 0: a compact one (the block forest below the block hashes
+ * is never allocated, see cdx_slot_compact).  CDX_ERR_ARG for a null ctx or out, CDX_ERR_ALLOC, CDX_ERR_CUDA.
+ *
+ * cdx_slot_builder_add_host: blocks [first_block, first_block + n_bytes / block_size) from pageable or pinned host memory.
+ * The call returns once the bytes have been copied out of `data`: the caller may reuse the buffer at once.  Statuses:
+ * CDX_ERR_ARG for a null builder or data; CDX_ERR_STATE after a successful finish; CDX_ERR_SIZE when n_bytes is zero or
+ * not a multiple of block_size; CDX_ERR_RANGE when the range leaves the slot (checked without overflow); CDX_ERR_STATE when
+ * a block of the range has been added before (the message names the smallest such block).  A refused add changes
+ * nothing.  CDX_ERR_CUDA: a device error of the tile this add completed; the builder then refuses every later call with
+ * CDX_ERR_STATE.
+ *
+ * Tiles and memory: the bytes go through four pinned chunks of a quarter tile each into two device tiles of
+ * tile_blocks = max(1, min(n_blocks, CODEX_COMMIT_TILE_MIB MiB / block_size)) blocks (256 MiB by default).  A chunk is
+ * copied to the device while the next one fills; a tile is hashed when it is full, in any block order: the cell sponge,
+ * the block trees in a scratch forest of the tile, and a scatter to the blocks' places in the handle, while the other
+ * device tile fills.  Adds that do not complete a tile launch no kernel.  Adds of several MiB are copied by several host
+ * threads, single blocks on the caller's thread.  When the pinned chunk an add needs is still in flight, the add waits for
+ * it: that is the only back-pressure.  The builder's memory is fixed by the tile size, whatever the slot size (about one
+ * tile of pinned host memory and two tiles plus their scratch forests on the device), besides the handle's own levels,
+ * which are allocated at create.  The builder has its own streams and staging buffers: other calls on the same context,
+ * and other builders, may run between two adds.
+ *
+ * cdx_slot_builder_finish: hashes the last partial tile, builds the slot tree and returns synchronised.  With blocks
+ * missing it is CDX_ERR_STATE, the message says how many and names the smallest; the builder stays usable (add them and
+ * finish again).  CDX_ERR_STATE after a successful finish, CDX_ERR_ARG for a null builder or out, CDX_ERR_CUDA.  On success
+ * the handle is byte for byte what cdx_slot_commit_host on the same bytes gives (every layer, the root, the export
+ * image), or with keep_forest == 0 what cdx_slot_commit_host followed by cdx_slot_compact gives (compact image,
+ * cdx_slot_device_bytes).  It belongs to the builder's context, works with every call a committed slot takes and is freed
+ * with cdx_slot_free; the builder's own buffers are released.  Checking the root against an expected root is the caller's
+ * job (cdx_slot_root), as for cdx_slot_import.
+ *
+ * cdx_slot_builder_free: accepted in every state and on NULL; an unfinished slot is discarded. */
+typedef struct cdx_slot_builder cdx_slot_builder;
+int cdx_slot_builder_create(cdx_ctx* ctx, uint64_t n_blocks, size_t cell_size, size_t block_size, int keep_forest, cdx_slot_builder** out);
+int cdx_slot_builder_add_host(cdx_slot_builder* b, uint64_t first_block, const uint8_t* data, size_t n_bytes);
+int cdx_slot_builder_finish(cdx_slot_builder* b, cdx_slot** out);
+void cdx_slot_builder_free(cdx_slot_builder* b);
+
 /* ---- all GPUs of one process -------------------------------------------------------------------------------
  * For a single-process host (the Nim cli, the C++ mirror): a group owns one context and one communicator rank per
  * device and runs every collective call on one worker thread per GPU.  Results are those of rank 0. */
